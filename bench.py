@@ -2,6 +2,7 @@
 """Benchmark of the batched game-dynamics hot path (BASELINE.json metric: batched env-steps/sec, Tron & Blokus 4-player).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload all|tron|blokus|ttt4|ttt2] [--impl b200|reference]
+                    [--dump-outputs DIR]
 
 ONE JSON line.  The top level is the headline workload (default: Tron 4-player 19x19, 65,536 batched envs --
 BASELINE.json configs[1], the configuration the metric is quoted on); with --workload all (the default) the other
@@ -15,24 +16,28 @@ How it is timed
   * L2: the configured batch (13.6 MB of Tron state) would sit in the 126 MB L2, so every rank holds G independent
     replicas of the batch (>= 4 x L2 of state in total) and consecutive steps cycle through them: each step's state
     comes from and goes back to HBM ("inputs larger than L2").  No flush kernel is needed.
-  * value: a K-step pass is a few hundred microseconds at the driver's K = 20, far too short to time on its own, so
-    the timed region is R back-to-back repetitions of the K-step sequence ("reps", chosen so that the region lasts
-    >= --min-ms, default 50 ms), captured in ONE CUDA graph (Python launch overhead would dominate a 4 us step) and
-    replayed once between two CUDA events on the launching stream.  The statistics row-sum (crl_stats_reduce) and the
-    NCCL all-reduce of the 32-slot vector follow on the same stream INSIDE the timed region; barrier + synchronize on
-    both sides; max over ranks.  ms_per_step = elapsed / (K * R).
+  * value: the timed region is exactly K = --steps steps, captured in ONE CUDA graph (Python launch overhead would
+    dominate a 4 us step) and replayed once between two CUDA events on the launching stream.  The statistics row-sum
+    (crl_stats_reduce) and the NCCL all-reduce of the 32-slot vector follow on the same stream INSIDE the timed
+    region; barrier + synchronize on both sides; max over ranks.  ms_per_step = elapsed / K.  A Tron step is ~4 us, so
+    a K that fills tens of milliseconds (several thousand steps) is needed before the region times the steps rather
+    than the launch of the graph and the statistics reduction; a workload whose region is shorter than
+    SHORT_REGION_MS carries a "warning".  K is at most MAX_STEPS.
   * e2e: through the public Python API for host-side policies (env.host_stepper: one CUDA-graph launch = H2D copy
-    of the pinned actions + step kernel + D2H copy of the result record into pinned memory), 8 environment batches
-    in flight, K * Re steps (>= --min-ms as well) so that the pipeline's ramp and drain are < 1 % of the region.
+    of the pinned actions + step kernel + D2H copy of the result record into pinned memory), 16 environment batches
+    in flight, K steps as well (the pipeline's ramp and drain are part of the region).
+  * --dump-outputs DIR: after the timed region, what its last step computed (the arrays a caller of that step
+    receives) is written as DIR/<workload>_<name>.npy.  Inputs are fixed seeds and the number of steps before the dump
+    is fixed by the arguments, so two builds run with the same arguments can be compared output for output.
   * roofline: algorithmic bytes per env-step (DESIGN.md section 4) x envs per launch / mean launch duration vs the
-    measured copy bandwidth in MEASURED_PEAKS.json; Blokus additionally against the integer issue roof (warp
+    copy bandwidth measured on the machine (MEASURED_PEAKS.json, not kept in the repository) or, without that file,
+    the 6 655 GB/s of a B200 at 1000 W (peaks()); Blokus additionally against the integer issue roof (warp
     instructions per step from the committed ncu count, INT_PEAKS.json).
   * cpu_baseline / --impl reference: the CPU oracle port (oracle/liboracle.so: plain-C restatement of the
     reference's Python -- the reference itself is Python and cannot travel to the GPU box) on all host cores.
 """
 import argparse
 import json
-import math
 import os
 import sys
 import threading
@@ -45,6 +50,9 @@ if ROOT not in sys.path:
 import numpy as np  # noqa: E402
 
 L2_BYTES = 126 << 20
+MAX_STEPS = 10000       # --steps bound: the timed graph and its single-chain twin hold K x launches nodes each (Blokus: 3
+                        # per step), and TTT-4p's next_state leg pre-records K x 1 MiB of actions
+SHORT_REGION_MS = 10.0  # a timed region shorter than this is reported with a warning: launch latency weighs in
 POLICY = "philox4x32-10 uniform random, auto-reset"
 
 WORKLOADS = {
@@ -70,7 +78,7 @@ def peaks():
     path = os.path.join(ROOT, "MEASURED_PEAKS.json")
     if os.path.exists(path):
         return float(json.load(open(path))["hbm_gbs"]), "measured (MEASURED_PEAKS.json hbm_gbs)"
-    return 6650.0, "fallback (B200_PROFILING.md)"
+    return 6655.0, "fallback: device-to-device copy of 4 GiB (read + write) on one B200 at its 1000 W power limit"
 
 
 def _load_json(*parts):
@@ -131,6 +139,24 @@ def graph_upload(graph, stream):
     the device inside the timed region.  (No kernel runs here; the timed steps are the graph's only execution.)"""
     from colosseumrl_b200 import _cudart
     _cudart.check(_cudart.rt().cudaGraphUpload(graph.raw_cuda_graph_exec(), stream.cuda_stream), "cudaGraphUpload")
+
+
+DUMP_ROWS = 1024    # environments per workload in --dump-outputs: with the widest row (Blokus valid lists, <= 4096 ids)
+                    # the files of all workloads stay below 64 MB
+
+
+def dump_outputs(dirname, workload, arrays):
+    """DIR/<workload>_<name>.npy for every array (batch first): the same seeded sample of DUMP_ROWS environments of
+    each, as float32 -- float64 where float32 would not hold every value exactly."""
+    os.makedirs(dirname, exist_ok=True)
+    rows = None
+    for name, t in arrays.items():
+        a = t.cpu().numpy() if hasattr(t, "cpu") else np.asarray(t)
+        if rows is None:
+            rows = np.sort(np.random.default_rng(0).choice(len(a), min(len(a), DUMP_ROWS), replace=False))
+        a = a[rows]
+        f = a.astype(np.float32)
+        np.save(os.path.join(dirname, "%s_%s.npy" % (workload, name)), f if np.array_equal(f, a) else a.astype(np.float64))
 
 
 # ---------------------------------------------------------------------------------------------- CPU arm
@@ -350,6 +376,12 @@ class TronWL:
         self.local_t[g] += 1
         env.step_(st, act, out=st)                             # in place; C-ABI crl_tron_step
 
+    def outputs(self, g):
+        """What the last step of replica g handed its caller: the new state (as the reference's observation) and the
+        step's result record (include/colosseum_b200.h)."""
+        env, st = self.envs[g], self.states[g]
+        return dict(env.state_to_observation(st, -1), result=st.result)
+
     def e2e_step(self, k):
         return _pipelined_e2e_step(self, k, 0)
 
@@ -410,6 +442,11 @@ class TTTWL:
             self.envs[g].rollout(self.states[g], self.local_t[g], 1)  # policy (in-kernel Philox) + step, one launch
         self.local_t[g] += 1
 
+    def outputs(self, g):
+        """The new state of replica g and its last step's result record."""
+        board, winner, mover = self.envs[g].state_arrays(self.states[g])
+        return {"board": board, "winner": winner, "mover": mover, "result": self.states[g].result}
+
     def e2e_step(self, k):
         return _pipelined_e2e_step(self, k, 0)
 
@@ -454,6 +491,17 @@ class BlokusWL:
         env.random_actions(self.valid[g], self.local_t[g], out=self.act[g])
         env.step_(st, self.act[g], out=st)                            # crl_blokus_step
         self.local_t[g] += 1
+
+    def outputs(self, g):
+        """The last step of replica g: the valid lists it was given (-1 past each list's end, which the legal kernel
+        leaves unwritten), the picked actions, the new state and the step's result record (byte 7 is unused)."""
+        env, st = self.envs[g], self.states[g]
+        counts, ids = self.valid[g]
+        n = counts.clamp(max=ids.shape[1])
+        col = self.torch.arange(ids.shape[1], device=ids.device)
+        ids = self.torch.where(col[None] < n[:, None], ids, -1)[:, :int(n.max())]
+        return dict(env.state_to_observation(st, -1), valid_counts=counts, valid_ids=ids, actions=self.act[g],
+                    result=st.result[:, :7])
 
     # e2e: a host-side policy needs two round trips per step -- it sees the list lengths (D2H), answers with an index
     # into the device-side list (H2D of one int32 per game; here: entry 0, pass if the list is empty), the step runs, the
@@ -640,26 +688,13 @@ def measure_b200(name, args, cx, with_cpu):
         torch.cuda.synchronize()
         return a.elapsed_time(b)
 
-    # size the timed region: a first K-step graph (one chain) gives the step time; R repetitions of the K-step sequence
-    # then fill >= --min-ms.  (These K steps are real steps of the same sequence: they double as warm-up.)
-    g0 = capture(k, K, 1)
-    (est,) = cx.max_over_ranks([max(timed_replay(g0) / K, 1e-4)])      # every rank must derive the same R
+    # K steps as ONE dependent chain (every launch waits for its predecessor): warm-up of graph replays before the timed
+    # one, and reported next to it when the timed graph has parallel chains
+    gs = capture(k, K, 1)
+    serial = timed_replay(gs) / K
     k += K
-    del g0
-    node_cap = 30000 // wl["launches"]
-    R = max(1, min(int(math.ceil(args.min_ms / (K * est))), max(1, node_cap // K)))
-    if args.reps > 0:
-        R = args.reps                              # (profiling: the same R as a plain run, whatever the profiler's clock says)
-    # for the report only: the same steps as ONE dependent chain (every launch waits for its predecessor)
-    serial, Rs = None, 0
-    if S > 1:
-        Rs = max(1, min(R // 2, max(1, node_cap // K)))
-        gs = capture(k, K * Rs, 1)
-        serial = timed_replay(gs) / (K * Rs)
-        k += K * Rs
-        del gs
-    n_timed = K * R
-    graph = capture(k, n_timed, S)
+    del gs
+    graph = capture(k, K, S)
     work.stats_env.stats_rows.zero_()              # count the timed steps only
     total_stats, _ = work.stats_env.all_reduce_stats(async_op=True)    # warm-up: NCCL communicator setup (zeros)
     torch.cuda.synchronize()
@@ -689,51 +724,45 @@ def measure_b200(name, args, cx, with_cpu):
     cx.barrier()
     torch.cuda.synchronize()
     wall = time.perf_counter() - wall0
-    k += n_timed
+    k += K
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, name, work.outputs((k - 1) % G))
     steps_ms = ev0.elapsed_time(ev1)
     dev_ms = ev0.elapsed_time(ev2)
     dev_ms_max, steps_ms_max = cx.max_over_ranks([dev_ms, steps_ms])
-    per_rank_step_ms = [x / (K * R) for x in cx.gather(steps_ms)]      # which GPU sets the max (B200s differ by a few % in HBM speed)
-    ms_per_step = dev_ms_max / n_timed
-    value = world * B * n_timed / (dev_ms_max * 1e-3)
-    step_ms = steps_ms_max / n_timed
+    per_rank_step_ms = [x / K for x in cx.gather(steps_ms)]      # which GPU sets the max (B200s differ by a few % in HBM speed)
+    ms_per_step = dev_ms_max / K
+    value = world * B * K / (dev_ms_max * 1e-3)
+    step_ms = steps_ms_max / K
     launch_ms = step_ms / wl["launches"]
 
     # ---- TTT only: next_state alone (crl_ttt_step with resident, pre-recorded actions) next to the fused policy + step
     next_state_only = None
     if name == "ttt4" and not args.no_e2e:
         work.mode = "next_state"
-        n2 = min(n_timed, 1024)
-        g2 = capture(k, n2, S)
-        (t2,) = cx.max_over_ranks([timed_replay(g2) / n2])
-        k += n2
+        g2 = capture(k, K, S)
+        (t2,) = cx.max_over_ranks([timed_replay(g2) / K])
+        k += K
         del g2
         work.mode, work.actions = "fused", None
-        next_state_only = {"ms_per_step": t2, "steps": n2, "algorithmic_bytes_per_env_step": 41,
+        next_state_only = {"ms_per_step": t2, "steps": K, "algorithmic_bytes_per_env_step": 41,
                            "note": "crl_ttt_step (next_state + fused valid-after mask) with resident actions recorded from the "
                                    "same random policy; 16 + 16 + 1 + 4 + 4 B per env-step"}
         work.stats_env.stats_rows.zero_()
 
-    # ---- end to end through the public API with host buffers: K x Re steps (>= --min-ms)
+    # ---- end to end through the public API with host buffers: K steps after W of warm-up
     if args.no_e2e:
         work.e2e_run = lambda k_, n_: 0
-    work.e2e_run(k, 3); k += 3
+    work.e2e_run(k, W); k += W
     torch.cuda.synchronize()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    probe_n = max(16, min(64, K))
-    t_ = time.perf_counter()
-    work.e2e_run(k, probe_n); k += probe_n
-    (est_e,) = cx.max_over_ranks([max((time.perf_counter() - t_) / probe_n * 1e3, 1e-3)])
-    Re = max(1, int(math.ceil(args.min_ms / (K * est_e))))
-    Ke = K * Re
-    torch.cuda.synchronize()
     cx.barrier()
     e0.record(stream)
-    work.e2e_run(k, Ke); k += Ke
+    work.e2e_run(k, K); k += K
     e1.record(stream)
     torch.cuda.synchronize()
     (e2e_ms,) = cx.max_over_ranks([e0.elapsed_time(e1)])
-    e2e_value = world * B * Ke / (e2e_ms * 1e-3)
+    e2e_value = world * B * K / (e2e_ms * 1e-3)
     clk = clocks.stop()
     # the same leg through the copy engines (memcpy H2D + kernel + memcpy D2H per step) next to the zero-copy transport
     e2e_copy = None
@@ -741,16 +770,15 @@ def measure_b200(name, args, cx, with_cpu):
         work.steppers, work.inflight = None, []
         work.stepper_kwargs = dict(work.stepper_kwargs, zero_copy=False)
         work.e2e_run(k, 48); k += 48
-        n_c = max(K, Ke // 3)
         torch.cuda.synchronize()
         cx.barrier()
         c0, c1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         c0.record(stream)
-        work.e2e_run(k, n_c); k += n_c
+        work.e2e_run(k, K); k += K
         c1.record(stream)
         torch.cuda.synchronize()
         (c_ms,) = cx.max_over_ranks([c0.elapsed_time(c1)])
-        e2e_copy = {"value": world * B * n_c / (c_ms * 1e-3), "steps": n_c,
+        e2e_copy = {"value": world * B * K / (c_ms * 1e-3), "steps": K,
                     "transport": "the same steps with explicit copies: one graph launch = memcpy H2D + step kernel + memcpy D2H"}
 
     out = None
@@ -767,7 +795,7 @@ def measure_b200(name, args, cx, with_cpu):
                "traffic": traffic, "peak_source": peak_src, "kernel": wl["kernel"],
                "algorithmic_bytes_per_env_step": bytes_per_step, "launch_ms": launch_ms,
                "note": "achieved = algorithmic bytes of the timed steps / device time of the steps (events around the graph)",
-               "single_chain": None if serial is None else
+               "single_chain": None if S == 1 else
                {"ms_per_step": serial, "frac": bytes_per_step * B / (serial * 1e-3) / 1e9 / peak,
                 "note": "same steps as one dependent chain (every launch waits for its predecessor, PDL only)"}}
         roofline = hbm
@@ -782,14 +810,14 @@ def measure_b200(name, args, cx, with_cpu):
                 roofline = issue
         out = {
             "metric": "batched env-steps/sec", "value": value, "unit": "env-steps/s", "n_gpus": world, "steps": K,
-            "warmup": W, "reps": R, "timed_steps": n_timed, "ms_per_step": ms_per_step, "higher_is_better": True,
+            "warmup": W, "timed_steps": K, "ms_per_step": ms_per_step, "higher_is_better": True,
             "scaling": args.scaling, "vs_baseline": None, "dtype": wl["dtype"], "data": "synthetic",
             "config": config_of(name, B),
             "method": {"l2": "inputs larger than L2: %d independent replicas of the batch per GPU (%.0f MB of state) "
                              "stepped round-robin, no flush kernel" % (G, G * per_replica / 1e6),
-                       "launch": "R = %d repetitions of the K-step sequence captured in one CUDA graph" % R +
+                       "launch": "the K timed steps captured in one CUDA graph" +
                                  ("" if S == 1 else ", the independent replicas spread over %d parallel chains (a replica's own steps stay ordered)" % S),
-                       "chains": S, "state_bytes_per_env": wl["state"], "warmup_extra_steps": extra_warm + K + K * Rs + desync,
+                       "chains": S, "state_bytes_per_env": wl["state"], "warmup_extra_steps": extra_warm + K + desync,
                        "phase_desync_steps": desync,
                        "timed_region_ms": dev_ms_max, "steps_ms": steps_ms_max,
                        "stats_allreduce_ms": dev_ms_max - steps_ms_max,
@@ -797,15 +825,18 @@ def measure_b200(name, args, cx, with_cpu):
                        "parallelism": "env-sharded x%d, no data-path collective, 1 stats all-reduce inside the timed region" % world},
             "roofline": roofline,
             "e2e": {"value": e2e_value, "unit": "env-steps/s", "h2d_bytes_per_step": work.h2d,
-                    "d2h_bytes_per_step": work.d2h, "steps": Ke,
+                    "d2h_bytes_per_step": work.d2h, "steps": K,
                     "transport": getattr(work, "e2e_note", "one graph launch per step = memcpy H2D of the pinned actions + "
                                          "step kernel + memcpy D2H of the result record into pinned memory"),
                     "copy_engine": e2e_copy},
-            "gpu_launches": n_timed * wl["launches"] * world + world,
+            "gpu_launches": K * wl["launches"] * world + world,
             "clocks": clk,
             "wall_s_timed_region": wall,
             "episodes": int(stats[1]), "env_steps_counted": int(stats[0]),
         }
+        if dev_ms_max < SHORT_REGION_MS:
+            out["warning"] = ("timed region %.3f ms < %g ms: graph launch latency is a visible share of it; a larger "
+                              "--steps measures the steady state" % (dev_ms_max, SHORT_REGION_MS))
         if with_cpu:
             out["cpu_baseline"] = cpu_baseline(name)
     # release this workload's device memory before the next one
@@ -827,30 +858,34 @@ def measure_ttt2(args, cx):
     rng = random.Random(0)
 
     def play(n):
-        done, state, players = 0, None, None
-        while done < n:
+        """n steps from a fresh game; returns what the last next_state call returned."""
+        state, players = None, None
+        for _ in range(n):
             if state is None:
                 state, players = env.new_state()
             p = players[0]
             a = rng.choice(env.valid_actions(state, p))
-            state, players, _, terminal, _ = env.next_state(state, players, [a])
-            done += 1
+            last = env.next_state(state, players, [a])
+            state, players, _, terminal, _ = last
             if terminal:
                 state = None
-        return done
+        return last
 
     play(max(3, args.warmup))
     torch.cuda.synchronize()
-    n = max(args.steps, 200)
+    n = args.steps
     t0 = time.perf_counter()
-    play(n)
+    (board, winner), players, rewards, terminal, _ = play(n)
     torch.cuda.synchronize()
     dt = time.perf_counter() - t0
     if cx.rank != 0:
         return None
+    if args.dump_outputs:                      # the winners list is [winner] or None: the state's winner says it already
+        dump_outputs(args.dump_outputs, "ttt2", {"board": [board], "winner": [-1 if winner is None else winner],
+                                                 "players": [players], "rewards": [rewards], "terminal": [terminal]})
     v = n / dt
     return {"metric": "batched env-steps/sec", "value": v, "unit": "env-steps/s", "n_gpus": 1, "steps": args.steps,
-            "warmup": args.warmup, "reps": 1, "timed_steps": n, "ms_per_step": dt / n * 1e3, "higher_is_better": True,
+            "warmup": args.warmup, "timed_steps": n, "ms_per_step": dt / n * 1e3, "higher_is_better": True,
             "scaling": "weak", "vs_baseline": None, "dtype": "u32", "data": "synthetic", "config": config_of("ttt2", 1),
             "method": {"note": "single-environment string-action adapter (colosseumrl_b200.single): valid_actions + "
                                "next_state per step = one host round trip (H2D action, crl_ttt_step, one D2H; the valid "
@@ -900,14 +935,15 @@ def main():
     _claim_stdout()
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=200)
+    ap.add_argument("--steps", type=int, default=200,
+                    help="timed steps of every measured leg of the b200 arm, 1 .. %d (the reference arm repeats each "
+                         "single-environment ttt2 step 1000 times, reported as reps)" % MAX_STEPS)
     ap.add_argument("--warmup", type=int, default=10)
     ap.add_argument("--workload", default="all", choices=["all"] + ORDER,
                     help="all (default): Tron is the headline line, the other BASELINE.json configurations are nested under `workloads`")
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
-    ap.add_argument("--min-ms", type=float, default=50.0,
-                    help="minimum length of every timed region; the K-step sequence is repeated to fill it")
-    ap.add_argument("--reps", type=int, default=0, help="force the number of repetitions R (profiling runs)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step of each workload computed to DIR/<workload>_<name>.npy")
     ap.add_argument("--profile-range", action="store_true",
                     help="bracket the timed graph replay with cudaProfilerStart/Stop (for ncu --profile-from-start off)")
     ap.add_argument("--no-e2e", action="store_true", help="profiling runs: skip the end-to-end leg")
@@ -922,6 +958,10 @@ def main():
     ap.add_argument("--streams", type=int, default=4, help="parallel chains of independent replicas inside the timed graph")
     ap.add_argument("--e2e-depth", type=int, default=0, help="environment batches in flight in the e2e leg (0 = default)")
     args = ap.parse_args()
+    if not 1 <= args.steps <= MAX_STEPS:
+        ap.error("--steps must be between 1 and %d" % MAX_STEPS)
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the b200 arm")
     args.warmup = max(args.warmup, 3)
     if args.e2e_depth > 0:
         global E2E_DEPTH

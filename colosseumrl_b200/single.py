@@ -62,8 +62,10 @@ class SingleEnvironment(_reference_base()):
     def observation_shape(self) -> Dict[str, tuple]:
         return self._b.observation_shape
 
-    def observation_names(self) -> List[str]:
-        return self._b.observation_names()
+    @classmethod
+    def observation_names(cls) -> List[str]:
+        """Static in the reference (callable on the class): the batched class's names."""
+        return cls._batched_class.observation_names()
 
     def compute_ranking(self, state, players: List[int], winners: List[int]) -> Dict[int, int]:
         """Default ranking (BaseEnvironment.py:173-195): winners 0, everybody else 1."""

@@ -20,7 +20,7 @@ for f in ("r2_bench_b", "r2_bench_ttt_nopdl", "r2_bench_tron_s1"):
         r = w.get("roofline") or {}
         sc = (r.get("single_chain") or (r.get("hbm") or {}).get("single_chain") or {})
         print(f, n, "value %.4g" % w["value"], "ms/step %.5f" % w["ms_per_step"], "frac %.3f" % (r.get("frac") or -1),
-              "single %.3f" % (sc.get("frac") or -1), "e2e %.4g" % w["e2e"]["value"], "reps", w.get("reps"), (w.get("cpu_baseline") or {}).get("value"))
+              "single %.3f" % (sc.get("frac") or -1), "e2e %.4g" % w["e2e"]["value"], "timed_steps", w.get("timed_steps"), (w.get("cpu_baseline") or {}).get("value"))
     show(d["config"]["workload"][:6], d)
     for n, w in (d.get("workloads") or {}).items():
         show(n, w)

@@ -24,7 +24,7 @@ for f in ("r2_bench_g1", "r2_bench_g2"):
         r = w.get("roofline") or {}
         sc = (r.get("single_chain") or (r.get("hbm") or {}).get("single_chain") or {})
         print(f, n, "value %.4g" % w["value"], "ms/step %.5f" % w["ms_per_step"], "frac %.3f" % (r.get("frac") or -1),
-              "single %.3f" % (sc.get("frac") or -1), "e2e %.4g" % w["e2e"]["value"], "reps", w.get("reps"), "allreduce_ms %.3f" % w["method"]["stats_allreduce_ms"])
+              "single %.3f" % (sc.get("frac") or -1), "e2e %.4g" % w["e2e"]["value"], "timed_steps", w.get("timed_steps"), "allreduce_ms %.3f" % w["method"]["stats_allreduce_ms"])
     show("tron", d)
     for n, w in (d.get("workloads") or {}).items():
         if n != "ttt2": show(n, w)

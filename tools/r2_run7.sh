@@ -14,16 +14,15 @@ NCU="ncu --clock-control none"
 for w in blokus ttt4; do
   python bench.py --workload $w --steps 20 --warmup 5 --no-cpu > $out/plain_${w}_$tag.json 2> $out/plain_${w}_$tag.err || echo "plain $w FAILED"
 done
-R() { python -c "import json; print(json.load(open('$out/plain_$1_$tag.json'))['reps'])"; }
 for w in blokus ttt4; do
   $NCU --profile-from-start off --metrics gpu__time_duration.sum,smsp__inst_executed.sum --csv --log-file $out/launches_${w}_$tag.csv \
-    python bench.py --workload $w --steps 20 --warmup 5 --no-cpu --no-e2e --reps $([ $w = blokus ] && R blokus || echo 2) --profile-range > $out/launches_${w}_$tag.log 2>&1 || echo "launch list $w FAILED"
+    python bench.py --workload $w --steps $([ $w = blokus ] && echo 420 || echo 40) --warmup 5 --no-cpu --no-e2e --profile-range > $out/launches_${w}_$tag.log 2>&1 || echo "launch list $w FAILED"
 done
 $NCU --set full --import-source on --profile-from-start off -k regex:ttt_rollout -s 30 -c 1 -o $out/prof_ttt_rollout_$tag -f \
-    python bench.py --workload ttt4 --steps 20 --warmup 5 --no-cpu --no-e2e --reps 4 --profile-range > $out/full_ttt_$tag.log 2>&1
+    python bench.py --workload ttt4 --steps 80 --warmup 5 --no-cpu --no-e2e --profile-range > $out/full_ttt_$tag.log 2>&1
 M=dram__bytes_read.sum,dram__bytes_write.sum,gpu__time_duration.sum,dram__throughput.avg.pct_of_peak_sustained_elapsed
 $NCU --graph-profiling graph --profile-from-start off --cache-control none --metrics $M --csv --log-file $out/graph_dram_ttt4_$tag.csv \
-    python bench.py --workload ttt4 --steps 50 --warmup 5 --no-cpu --no-e2e --reps 2 --profile-range > $out/graph_dram_ttt4_$tag.log 2>&1 || echo "graph dram ttt4 FAILED"
+    python bench.py --workload ttt4 --steps 100 --warmup 5 --no-cpu --no-e2e --profile-range > $out/graph_dram_ttt4_$tag.log 2>&1 || echo "graph dram ttt4 FAILED"
 # observe kernels, one capture per kernel
 for k in tron_observe blokus_observe ttt_observe; do
   $NCU --set full --import-source on -k regex:$k -c 2 -o $out/prof_${k}_$tag -f python tools/observe_probe.py > $out/full_${k}_$tag.log 2>&1

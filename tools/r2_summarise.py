@@ -67,7 +67,7 @@ def graph_dram(tag):
     lines = ["# Graph-level DRAM traffic of bench.py's timed graphs (`ncu --graph-profiling graph --cache-control none`)", "",
              "The whole timed CUDA graph is ONE profiled workload: its launches run back to back with the caches as they",
              "are (per-kernel captures flush the caches and serialise the launches, so write-backs that leave L2 after a",
-             "kernel ends are never counted there).  `steps` = --steps x --reps of the profiled command (tools/r2_profile.sh).", "",
+             "kernel ends are never counted there).  `steps` = --steps of the profiled command (tools/r2_profile.sh).", "",
              "| graph | steps | DRAM read / step | DRAM write / step | read + write / step | algorithmic / step | graph time / step (under ncu) | dram__throughput |",
              "|---|---|---|---|---|---|---|---|"]
     alg = {"tron": 424 * 65536, "ttt4": 36 * (1 << 20)}
