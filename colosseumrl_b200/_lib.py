@@ -62,6 +62,7 @@ SIGNATURES = {
     "crl_blokus_is_valid": (_int, [_vp, _int, _vp, _vp, _i64, _int, _vp]),
     "crl_blokus_step": (_int, [_vp, _vp, _vp, _vp, _vp, _i64, _int, _vp]),
     "crl_blokus_policy_random": (_int, [_vp, _vp, _i32, _vp, _u64, _u64, _u32, _i64, _vp]),
+    "crl_blokus_rollout": (_int, [_vp, _vp, _vp, _u64, _u64, _u32, _int, _i64, _vp]),
     "crl_blokus_pick": (_int, [_vp, _vp, _i32, _vp, _vp, _i64, _vp]),
     "crl_blokus_observe": (_int, [_vp, _int, _vp, _vp, _vp, _vp, _i64, _vp]),
     "crl_blokus_pack": (_int, [_vp, _vp, _vp, _vp, _vp, _i64, _vp]),

@@ -199,6 +199,19 @@ class BatchedBlokusEnvironment(BatchedBaseEnvironment):
                                               meta.data_ptr(), self.batch, self._stream))
         return st
 
+    def rollout(self, state: BlokusBatchState, step0: int, K: int) -> BlokusBatchState:
+        """K uniform-random-policy steps (steps step0 .. step0 + K - 1 of this env's seed and env ids) in one launch,
+        state updated in place; the last step's record goes to state.result and the statistics to `stats`.  Finished
+        games are always restarted, whatever `auto_reset` says.  Equal to K x valid_actions -> random_actions -> step_
+        with auto-reset whenever every list fits `capacity`: the pick is drawn over the full list, which is never
+        stored."""
+        if state.result is None:
+            state.result = self._new_result((self.batch, 8))
+        self._check(self._lib.crl_blokus_rollout(state.packed.data_ptr(), state.result.data_ptr(), self._stats_ptr,
+                                                 self.seed, self.first_env_id, int(step0), int(K), self.batch,
+                                                 self._stream))
+        return state
+
     def random_actions(self, valid, step: int, out: Optional[torch.Tensor] = None) -> torch.Tensor:
         counts, ids = valid
         out = out if out is not None else torch.empty((self.batch,), dtype=torch.int32, device=self.device)

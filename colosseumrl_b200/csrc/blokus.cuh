@@ -282,7 +282,14 @@ __device__ __forceinline__ int blk_any_move(BlkSmem &sm, int c, int round, uint3
 // byte per group (5 hit bits), so ONE SWAR popcount and ONE shuffle scan position all hits of up to 16 anchors:
 // lane order (a, o) followed by k IS the reference's order (anchor row-major -> orientation -> shift), and the action
 // id is anchor code + piece * 16000 + o * 5 + k.  Each lane then stores its own <= 5 ids of a group.
-template <bool PENT>
+// MODE (compile time):
+//   BLK_STORE   store the ids into out[base..cap) and return base + the piece's count;
+//   BLK_COUNT   return base + the piece's count: no scan and no store, one popcount per lane and chunk and ONE warp
+//               reduction per piece;
+//   BLK_SELECT  return the id at index `cap` of the piece's own list (base 0, out unused; cap < the piece's count):
+//               the store phase with the stores replaced by "the lane whose range holds index cap keeps that id".
+enum { BLK_STORE = 0, BLK_COUNT = 1, BLK_SELECT = 2 };
+template <bool PENT, int MODE = BLK_STORE>
 __device__ __forceinline__ int blk_emit_piece(BlkSmem &sm, uint32_t nemask, int p, int na, int lane, int base,
                                               int32_t *__restrict__ out, int cap) {
     // nemask: the non-empty flags the piece's table entries index (`ne`, or its pentomino group's `ne5`)
@@ -296,6 +303,7 @@ __device__ __forceinline__ int blk_emit_piece(BlkSmem &sm, uint32_t nemask, int 
     const uint32_t f0 = e0.x, f1 = e0.y, f2 = e0.z, f3 = e0.w, f4 = e1.x;          // row offsets, bytes
     const uint32_t c0 = e1.y, c1 = e1.z, c2 = e1.w, c3 = e2.x, c4 = e2.y;          // column constants
     const int val00 = p * 16000 + o * 5;
+    int cnt = 0, sel = -1;                                   // BLK_COUNT: the lane's hits; BLK_SELECT: the id found
 #define BLK_TEST(fk, ck) hh = __funnelshift_r(hh, __funnelshift_r(*(const uint32_t *)(fb + ((fk) + row)), 0u, w + (ck)), 1)
 #pragma unroll 1
     for (int a0 = 0; a0 < na; a0 += 16) {                    // chunks of four groups (one chunk in practice: ~8 anchors)
@@ -322,6 +330,10 @@ __device__ __forceinline__ int blk_emit_piece(BlkSmem &sm, uint32_t nemask, int 
             }
         }
         hh = v ? hh : 0u;                                    // byte g = hits of (anchor a0 + 4 g + a, o), bit k = shift k
+        if (MODE == BLK_COUNT) {
+            cnt += __popc(hh);
+            continue;
+        }
         if (!__any_sync(0xffffffffu, hh != 0u)) continue;
         uint32_t cc = hh - ((hh >> 1) & 0x55555555u);        // per-byte popcount
         cc = (cc & 0x33333333u) + ((cc >> 2) & 0x33333333u);
@@ -338,10 +350,14 @@ __device__ __forceinline__ int blk_emit_piece(BlkSmem &sm, uint32_t nemask, int 
             uint32_t h = (hh >> (8 * g)) & 0xffu;
             int pos = base + (int)((excl >> (8 * g)) & 0xffu);
             base += tg;
-            if (careful)                                     // drop the ids that do not fit (the count stays complete)
+            if (MODE == BLK_STORE && careful)                // drop the ids that do not fit (the count stays complete)
                 while (h != 0u && __popc(h) > max(cap - pos, 0)) h &= ~(0x80000000u >> __clz((int)h));
             const uint32_t w = wg[g];
             const int val0 = (int)(w >> 9) * 200 + (int)(w & 31u) * 40 + val00;      // (y * 20 + x) * 40 + ...
+            if (MODE == BLK_SELECT) {                        // ids pos .. pos + popc(h) - 1 are this lane's
+                if (pos <= cap && cap < pos + __popc(h)) sel = val0 + (int)__fns(h, 0u, cap - pos + 1);
+                continue;
+            }
             // (32-bit running index: a 64-bit running pointer costs predicated 64-bit adds and moves per store)
             if (h & 1u) st_global_u32(out + pos++, val0);
             if (h & 2u) st_global_u32(out + pos++, val0 + 1);
@@ -349,43 +365,86 @@ __device__ __forceinline__ int blk_emit_piece(BlkSmem &sm, uint32_t nemask, int 
             if (h & 8u) st_global_u32(out + pos++, val0 + 3);
             if (h & 16u) st_global_u32(out + pos, val0 + 4);
         }
+        if (MODE == BLK_SELECT && base > cap) break;        // (warp-uniform) found
     }
 #undef BLK_TEST
+    if (MODE == BLK_COUNT) return base + __reduce_add_sync(0xffffffffu, cnt);
+    if (MODE == BLK_SELECT) return (int)__reduce_or_sync(0xffffffffu, (uint32_t)(sel + 1)) - 1;   // one lane holds it
     return base;
 }
 
-// Enumerate the legal moves of player c holding `inv` on the board in sm.st: action ids in the reference's order
-// into out[0..cap), returns the full count.
+// the monomino's id at index i of its list after round 0 (anchor i >> 3, orientation i & 7, shift 0; see below)
+__device__ __forceinline__ int blk_monomino_id(const BlkSmem &sm, int i) {
+    const uint32_t w = sm.anch[i >> 3];
+    return (int)(w >> 9) * 200 + (int)(w & 31u) * 40 + 5 * (i & 7);
+}
+
+// Enumerate the legal moves of player c holding `inv` on the board in sm.st.
+//   MODE == BLK_STORE:  action ids in the reference's order into out[0..cap), returns the full count.
+//   MODE == BLK_SELECT: a uniform random pick without the list.  A count pass (the same enumeration without the store
+//     phase; lane p keeps the count of piece p) gives the length n; for n > 0 the pick is the id at index rnd % n of
+//     the full list, which a warp scan over the per-piece counts turns into a piece p* and an index into its ids, and
+//     a select pass over p* alone finds.  *pick = that id (-1 if n == 0); returns n.  out / cap are unused.
+template <int MODE = BLK_STORE>
 __device__ __forceinline__ int blk_enumerate(BlkSmem &sm, int c, int round, uint32_t inv, int lane,
-                                             int32_t *__restrict__ out, int cap) {
+                                             int32_t *__restrict__ out, int cap, uint32_t rnd = 0u, int *pick = nullptr) {
+    constexpr int EMIT = MODE == BLK_STORE ? BLK_STORE : BLK_COUNT;
     inv = __reduce_or_sync(0xffffffffu, inv);                // same in every lane
+    if (MODE == BLK_SELECT) *pick = -1;
     const int na = blk_allowed_and_anchors<true>(sm, c, round, lane);
     if (na == 0 || inv == 0u) return 0;
     uint32_t ne = blk_tree_root(sm, lane);
     ne |= blk_tree_pass_le4(sm, ne, inv, lane);
-    int base = 0;
+    int base = 0, pcount = 0, glast = -1;                    // (BLK_SELECT) count of piece `lane`, last group built
+    uint32_t ne5last = 0u;
     uint32_t small = inv & ((1u << BLK_GROUP_P0[0]) - 1u);                                   // pieces of <= 4 cells
     if ((small & 1u) && round != 0) {
         // the monomino needs no test after round 0: every anchor is an allowed cell (ANC = A & D4), so it fits on each
         // in all 8 orientations (k = 0) -- ids (y * 20 + x) * 40 + 5 o in anchor order, written 32 at a time
-        for (int i = lane; i < 8 * na; i += 32) {
-            const uint32_t w = sm.anch[i >> 3];
-            if (i < cap) st_global_u32(out + i, (int)(w >> 9) * 200 + (int)(w & 31u) * 40 + 5 * (i & 7));
-        }
+        if (MODE == BLK_STORE)
+            for (int i = lane; i < 8 * na; i += 32)
+                if (i < cap) st_global_u32(out + i, blk_monomino_id(sm, i));
+        if (lane == 0) pcount = 8 * na;
         base = 8 * na;
         small &= ~1u;
     }
 #pragma unroll 1
-    for (uint32_t rest = small; rest; rest &= rest - 1u)
-        base = blk_emit_piece<false>(sm, ne, __ffs((int)rest) - 1, na, lane, base, out, cap);
+    for (uint32_t rest = small; rest; rest &= rest - 1u) {
+        const int p = __ffs((int)rest) - 1, next = blk_emit_piece<false, EMIT>(sm, ne, p, na, lane, base, out, cap);
+        if (lane == p) pcount = next - base;
+        base = next;
+    }
 #pragma unroll 1
     for (int g = 0; g < BLK_NGROUP; g++) {                                                   // pentominoes, group by group
         uint32_t rest = inv & ((1u << BLK_GROUP_P0[g + 1]) - (1u << BLK_GROUP_P0[g]));
         if (rest == 0u) continue;
         const uint32_t ne5 = blk_tree_group(sm, g, ne, inv, lane);
+        glast = g;
+        ne5last = ne5;
         if (ne5 == 0u) continue;
 #pragma unroll 1
-        for (; rest; rest &= rest - 1u) base = blk_emit_piece<true>(sm, ne5, __ffs((int)rest) - 1, na, lane, base, out, cap);
+        for (; rest; rest &= rest - 1u) {
+            const int p = __ffs((int)rest) - 1, next = blk_emit_piece<true, EMIT>(sm, ne5, p, na, lane, base, out, cap);
+            if (lane == p) pcount = next - base;
+            base = next;
+        }
+    }
+    if (MODE == BLK_STORE || base == 0) return base;
+    // pick: piece p* = the first piece whose inclusive prefix count exceeds r, j = r - the ids before p*
+    const uint32_t r = rnd % (uint32_t)base;
+    int incl = pcount;
+#pragma unroll
+    for (int d = 1; d < 32; d <<= 1) incl = (int)warp_scan_step((uint32_t)incl, d);
+    const int ps = __popc(__ballot_sync(0xffffffffu, (uint32_t)incl <= r));
+    const int j = (int)r - __shfl_sync(0xffffffffu, incl - pcount, ps);
+    if (ps == 0 && round != 0) {
+        *pick = blk_monomino_id(sm, j);
+    } else if (ps < BLK_GROUP_P0[0]) {
+        *pick = blk_emit_piece<false, BLK_SELECT>(sm, ne, ps, na, lane, 0, out, j);   // the <= 4-cell boards are intact
+    } else {
+        const int g = BLK_PIECE_GROUP[ps];
+        if (g != glast) ne5last = blk_tree_group(sm, g, ne, inv, lane);          // a later group overwrote its boards
+        *pick = blk_emit_piece<true, BLK_SELECT>(sm, ne5last, ps, na, lane, 0, out, j);
     }
     return base;
 }
@@ -476,11 +535,97 @@ blokus_legal_kernel(const uint4 *__restrict__ st, int32_t *__restrict__ counts, 
 }
 
 // ---- next_state: one warp per game.
+// BlkStepOut: what one next_state produced, every field warp-uniform.
 // result record, 8 bytes: int8 reward | u8 flags (1 terminal, 2 illegal action, 4 placed) | u8 winners mask |
 //                         u8 ranking bits (bit p = rank of p: winners 0, others 1) | u8 next mover |
 //                         u8 next-players mask (1 << next mover) | u8 terminal (0 / 1) | 1 unused
 //                         (the last two repeat information as plain bytes so that the host layer returns VIEWS of the
 //                         record -- next_state's new_players and terminal -- without any element-wise decoding launch)
+struct BlkStepOut {
+    int mover, reward, terminal, error, placed, winners;
+    uint32_t scores, ep_len;                                 // the new scores (one byte per player), episode steps
+};
+__device__ __forceinline__ uint2 blk_result(const BlkStepOut &o) {
+    const uint32_t rank = 0xfu & ~(uint32_t)o.winners;
+    const int nmover = (o.mover + 1) & 3;
+    return make_uint2(((uint32_t)o.reward & 0xffu) | (uint32_t)(o.terminal | o.error << 1 | o.placed << 2) << 8 |
+                          (uint32_t)o.winners << 16 | rank << 24,
+                      (uint32_t)nmover | (1u << nmover) << 8 | (uint32_t)o.terminal << 16);
+}
+
+// next_state of the game in sm.st with action id `aid` (-1 = pass): the new state is committed into sm.st (the caller
+// stores it).  `zeroed`: the FIT boards have been zeroed in this kernel (blk_any_move zeroes them on first use).
+__device__ __forceinline__ BlkStepOut blk_step_apply(BlkSmem &sm, int aid, int lane, bool &zeroed) {
+    const uint32_t meta = sm.st[85];
+    const int round = (int)(meta & 0xffu), mover = (int)(meta >> 8 & 3u);
+    uint32_t inv[4] = {sm.st[80], sm.st[81], sm.st[82], sm.st[83]};
+    uint32_t scores = sm.st[84];
+    uint32_t new_row = lane < 20 ? sm.st[20 * mover + lane] : 0u;
+    int error = 0, placed = 0;
+    if (aid >= 0) {
+        uint32_t minv = 0, add;
+#pragma unroll
+        for (int q = 0; q < 4; q++) minv |= (q == mover) ? inv[q] : 0u;
+        int pc, size;
+        const bool legal = blk_validate(sm, mover, round, minv, aid, lane, add, pc, size);
+        if (legal) {
+            placed = 1;
+            new_row |= add;                                                     // Board.update_board
+            const uint32_t left = minv & ~(1u << pc);
+            int gain = size + (left == 0 ? (pc == 0 ? 20 : 15) : 0);            // AI.update_player (ai.py:44-54)
+#pragma unroll
+            for (int q = 0; q < 4; q++) {
+                if (q == mover) {
+                    inv[q] = left;
+                    scores = (scores & ~(0xffu << (8 * q))) | ((((scores >> (8 * q)) & 0xffu) + gain) & 0xffu) << (8 * q);
+                }
+            }
+        } else {
+            error = 1;                                                          // illegal id: flagged, applied as a pass
+        }
+    }
+    // terminal test on the OLD board / OLD round with the NEW inventories (BlokusEnvironment.py:424, SURVEY B6)
+    // `any` is order-independent; start with the players that have not moved yet this round (in round 0 the
+    // ones that already moved have an occupied corner and would need a full, fruitless scan) and end with the mover.
+    int any = 0;
+    uint32_t stuck = sm.st[87] & 15u;
+#pragma unroll 1
+    for (int j = 1; j <= 4 && !any; j++) {
+        const int q = (mover + j) & 3;
+        if (stuck >> q & 1u) continue;                                          // known: no move any more
+        uint32_t iq = 0;
+#pragma unroll
+        for (int r = 0; r < 4; r++) iq |= (r == q) ? inv[r] : 0u;
+        any = blk_any_move(sm, q, round, iq, lane, zeroed);
+        if (!any && j < 4 && round >= 1) stuck |= 1u << q;                      // (see the layout comment, w[87])
+    }
+    const int terminal = !any;
+    int reward = 0, winners = 0;
+    int sc[4] = {(int)(scores & 0xff), (int)(scores >> 8 & 0xff), (int)(scores >> 16 & 0xff), (int)(scores >> 24)};
+    if (terminal) {                                                             // :425-440
+        int mx = max(max(sc[0], sc[1]), max(sc[2], sc[3]));                     // max_score starts at 0, scores >= 0
+        int ms = 0;
+#pragma unroll
+        for (int q = 0; q < 4; q++) ms |= (q == mover) ? sc[q] : 0;
+#pragma unroll
+        for (int q = 0; q < 4; q++) {
+            winners |= (sc[q] == mx) ? (1 << q) : 0;
+            reward += (sc[q] < ms || (sc[q] == ms && q < mover)) ? 1 : 0;       // index in the stable ascending sort
+        }
+    }
+    const int nround = round + (mover == 3 ? 1 : 0), nmover = (mover + 1) & 3;  // :446-449
+    const uint32_t ep_len = sm.st[86] + 1u;
+    // commit into the shared copy (the caller stores it with 22 x 128-bit lanes)
+    __syncwarp();
+    if (lane < 20) sm.st[20 * mover + lane] = new_row;
+    if (lane < 4) sm.st[80 + lane] = lane == 0 ? inv[0] : lane == 1 ? inv[1] : lane == 2 ? inv[2] : inv[3];
+    if (lane == 4) sm.st[84] = scores;
+    if (lane == 5) sm.st[85] = (uint32_t)(nround & 0xff) | (uint32_t)nmover << 8 | (uint32_t)terminal << 16;
+    if (lane == 6) sm.st[86] = ep_len;
+    if (lane == 7) sm.st[87] = stuck;
+    return BlkStepOut{mover, reward, terminal, error, placed, winners, scores, ep_len};
+}
+
 __global__ void __launch_bounds__(32 * BLK_WARPS)
 blokus_step_kernel(const uint4 *__restrict__ in, uint4 *__restrict__ outst, const int32_t *__restrict__ actions,
                    uint2 *__restrict__ result, crl_u64 *stats, long long B, int flags) {
@@ -495,93 +640,23 @@ blokus_step_kernel(const uint4 *__restrict__ in, uint4 *__restrict__ outst, cons
         blk_load(sm, in, g, lane);
         bool zeroed = false;
         if ((flags & CRL_FLAG_AUTO_RESET) && (sm.st[85] >> 16 & 1u)) blk_new_state(sm, lane);
-        const uint32_t meta = sm.st[85];
-        const int round = (int)(meta & 0xffu), mover = (int)(meta >> 8 & 3u);
-        const int aid = actions[g];
-        uint32_t inv[4] = {sm.st[80], sm.st[81], sm.st[82], sm.st[83]};
-        uint32_t scores = sm.st[84];
-        uint32_t new_row = lane < 20 ? sm.st[20 * mover + lane] : 0u;
-        int error = 0, placed = 0;
-        if (aid >= 0) {
-            uint32_t minv = 0, add;
-#pragma unroll
-            for (int q = 0; q < 4; q++) minv |= (q == mover) ? inv[q] : 0u;
-            int pc, size;
-            const bool legal = blk_validate(sm, mover, round, minv, aid, lane, add, pc, size);
-            if (legal) {
-                placed = 1;
-                new_row |= add;                                                     // Board.update_board
-                const uint32_t left = minv & ~(1u << pc);
-                int gain = size + (left == 0 ? (pc == 0 ? 20 : 15) : 0);            // AI.update_player (ai.py:44-54)
-#pragma unroll
-                for (int q = 0; q < 4; q++) {
-                    if (q == mover) {
-                        inv[q] = left;
-                        scores = (scores & ~(0xffu << (8 * q))) | ((((scores >> (8 * q)) & 0xffu) + gain) & 0xffu) << (8 * q);
-                    }
-                }
-            } else {
-                error = 1;                                                          // illegal id: flagged, applied as a pass
-            }
-        }
-        // terminal test on the OLD board / OLD round with the NEW inventories (BlokusEnvironment.py:424, SURVEY B6)
-        // `any` is order-independent; start with the players that have not moved yet this round (in round 0 the
-        // ones that already moved have an occupied corner and would need a full, fruitless scan) and end with the mover.
-        int any = 0;
-        uint32_t stuck = sm.st[87] & 15u;
-#pragma unroll 1
-        for (int j = 1; j <= 4 && !any; j++) {
-            const int q = (mover + j) & 3;
-            if (stuck >> q & 1u) continue;                                          // known: no move any more
-            uint32_t iq = 0;
-#pragma unroll
-            for (int r = 0; r < 4; r++) iq |= (r == q) ? inv[r] : 0u;
-            any = blk_any_move(sm, q, round, iq, lane, zeroed);
-            if (!any && j < 4 && round >= 1) stuck |= 1u << q;                      // (see the layout comment, w[87])
-        }
-        const int terminal = !any;
-        int reward = 0, winners = 0;
-        int sc[4] = {(int)(scores & 0xff), (int)(scores >> 8 & 0xff), (int)(scores >> 16 & 0xff), (int)(scores >> 24)};
-        if (terminal) {                                                             // :425-440
-            int mx = max(max(sc[0], sc[1]), max(sc[2], sc[3]));                     // max_score starts at 0, scores >= 0
-            int ms = 0;
-#pragma unroll
-            for (int q = 0; q < 4; q++) ms |= (q == mover) ? sc[q] : 0;
-#pragma unroll
-            for (int q = 0; q < 4; q++) {
-                winners |= (sc[q] == mx) ? (1 << q) : 0;
-                reward += (sc[q] < ms || (sc[q] == ms && q < mover)) ? 1 : 0;       // index in the stable ascending sort
-            }
-        }
-        const int nround = round + (mover == 3 ? 1 : 0), nmover = (mover + 1) & 3;  // :446-449
-        const uint32_t ep_len = sm.st[86] + 1u;
-        // commit into the shared copy, then store with 22 x 128-bit lanes
-        __syncwarp();
-        if (lane < 20) sm.st[20 * mover + lane] = new_row;
-        if (lane < 4) sm.st[80 + lane] = lane == 0 ? inv[0] : lane == 1 ? inv[1] : lane == 2 ? inv[2] : inv[3];
-        if (lane == 4) sm.st[84] = scores;
-        if (lane == 5) sm.st[85] = (uint32_t)(nround & 0xff) | (uint32_t)nmover << 8 | (uint32_t)terminal << 16;
-        if (lane == 6) sm.st[86] = ep_len;
-        if (lane == 7) sm.st[87] = stuck;
+        const BlkStepOut o = blk_step_apply(sm, actions[g], lane, zeroed);
         blk_store(sm, outst, g, lane);
         if (lane == 0) {
-            const uint32_t rank = 0xfu & ~(uint32_t)winners;
-            result[g] = make_uint2(((uint32_t)reward & 0xffu) | (uint32_t)(terminal | error << 1 | placed << 2) << 8 |
-                                       (uint32_t)winners << 16 | rank << 24,
-                                   (uint32_t)nmover | (1u << nmover) << 8 | (uint32_t)terminal << 16);
+            result[g] = blk_result(o);
             if (stats) {
                 atomicAdd(&sm_stat[ST_STEPS], 1);
-                if (error) atomicAdd(&sm_stat[ST_ERRORS], 1);
-                if (reward) atomicAdd(&sm_stat[ST_REWARD], (mover + 1) * reward);
-                if (terminal) {
+                if (o.error) atomicAdd(&sm_stat[ST_ERRORS], 1);
+                if (o.reward) atomicAdd(&sm_stat[ST_REWARD], (o.mover + 1) * o.reward);
+                if (o.terminal) {
                     atomicAdd(&sm_stat[ST_EPISODES], 1);
-                    atomicAdd(&sm_stat[ST_EPLEN], (int)ep_len);
-                    if (!winners) atomicAdd(&sm_stat[ST_NOWIN], 1);
+                    atomicAdd(&sm_stat[ST_EPLEN], (int)o.ep_len);
+                    if (!o.winners) atomicAdd(&sm_stat[ST_NOWIN], 1);
 #pragma unroll
                     for (int q = 0; q < 4; q++) {
-                        if (winners >> q & 1) atomicAdd(&sm_stat[ST_WINS + q], 1);
+                        if (o.winners >> q & 1) atomicAdd(&sm_stat[ST_WINS + q], 1);
                         else atomicAdd(&sm_stat[ST_RANK + q], 1);
-                        atomicAdd(&sm_stat[ST_SCORE + q], sc[q]);
+                        atomicAdd(&sm_stat[ST_SCORE + q], (int)(q == 3 ? o.scores >> 24 : o.scores >> (8 * q) & 0xffu));
                     }
                 }
             }
@@ -599,6 +674,57 @@ __global__ void blokus_policy_random_kernel(const int32_t *__restrict__ counts, 
     int n = min(counts[g], cap);
     uint4 r = env_words(seed, first_env + (crl_u64)g, step, CRL_TAG_BLOKUS);
     actions[g] = n > 0 ? ids[g * cap + (long long)(r.x % (uint32_t)n)] : -1;
+}
+
+// ---- K fused random-policy steps with auto-reset: one warp per game, the game stays in shared memory for all K steps.
+// Step t is K x (legal kernel, player -1, auto-reset -> policy_random(step0 + t) -> step kernel, auto-reset) with the
+// list never materialised: blk_enumerate<BLK_SELECT> counts the mover's ids and finds the one at index
+// philox(env, step0 + t, tag 2)[0] % n of the FULL list, blk_step_apply applies it.  Statistics: lane s accumulates
+// slot s of this game in 64 bits (no overflow for any K) and adds it to the CTA's row once.
+__global__ void __launch_bounds__(32 * BLK_WARPS)
+blokus_rollout_kernel(uint4 *__restrict__ st, uint2 *__restrict__ result, crl_u64 *stats, long long B, crl_u64 seed,
+                      crl_u64 first_env, uint32_t step0, int K) {
+    __shared__ BlkSmem smem[BLK_WARPS];
+    const int lane = BLK_WARPS == 1 ? (int)threadIdx.x : (int)(threadIdx.x & 31), wid = BLK_WARPS == 1 ? 0 : (int)(threadIdx.x >> 5);
+    const long long g = (long long)blockIdx.x * BLK_WARPS + wid;
+    if (g >= B) return;
+    BlkSmem &sm = smem[wid];
+    blk_load(sm, st, g, lane);
+    // Zeroed once: the passes rewrite rows 0..19 of the boards they build and every read of a board is masked by the
+    // non-empty flags of the current pass, so a stale board from an earlier step is never used.
+    blk_zero_fit(sm, lane);
+    bool zeroed = true;
+    crl_u64 acc = 0;
+    uint2 rec = make_uint2(0u, 0u);
+#pragma unroll 1
+    for (int t = 0; t < K; t++) {
+        __syncwarp();                                        // the previous step's commit (and the zeroing) is visible
+        if (sm.st[85] >> 16 & 1u) blk_new_state(sm, lane);
+        const uint32_t meta = sm.st[85];
+        const int c = (int)(meta >> 8 & 3u);
+        int aid = -1, n = 0;
+        if (!(sm.st[87] >> c & 1u)) {                        // not known to be stuck (w[87]): enumerate
+            const uint32_t r = env_words(seed, first_env + (crl_u64)g, step0 + (uint32_t)t, CRL_TAG_BLOKUS).x;
+            n = blk_enumerate<BLK_SELECT>(sm, c, (int)(meta & 0xffu), sm.st[80 + c], lane, nullptr, 0, r, &aid);
+        }
+        const BlkStepOut o = blk_step_apply(sm, aid, lane, zeroed);
+        rec = blk_result(o);
+        if (stats) {                                         // the slots the legal and step kernels add
+            int v = lane == ST_STEPS ? 1 : lane == ST_NVALID ? n : lane == ST_ERRORS ? o.error
+                  : lane == ST_REWARD ? (o.mover + 1) * o.reward : 0;
+            if (o.terminal) {
+                const int q = (lane - ST_WINS) & 3, sq = (lane - ST_SCORE) & 3, rq = (lane - ST_RANK) & 3;
+                v += lane == ST_EPISODES ? 1 : lane == ST_EPLEN ? (int)o.ep_len : lane == ST_NOWIN ? (o.winners == 0)
+                   : (lane >= ST_WINS && lane < ST_WINS + 4) ? (o.winners >> q & 1)
+                   : (lane >= ST_SCORE && lane < ST_SCORE + 4) ? (int)(o.scores >> (8 * sq) & 0xffu)
+                   : (lane >= ST_RANK && lane < ST_RANK + 4) ? (~o.winners >> rq & 1) : 0;
+            }
+            acc += (crl_u64)(long long)v;
+        }
+    }
+    blk_store(sm, st, g, lane);
+    if (result && lane == 0) result[g] = rec;
+    if (stats && acc != 0) atomicAdd(stats + (blockIdx.x & (CRL_STAT_ROWS - 1)) * CRL_NSTAT + lane, acc);
 }
 
 // a host-side policy's choice: actions[g] = the choice[g]-th entry of game g's valid list, pass (-1) if choice[g] is

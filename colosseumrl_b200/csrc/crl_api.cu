@@ -759,6 +759,17 @@ int crl_blokus_policy_random(const int32_t *counts, const int32_t *action_ids, i
     return check_launch("blokus_policy_random_kernel");
 }
 
+int crl_blokus_rollout(void *state, uint8_t *result, int64_t *stats, uint64_t seed, uint64_t first_env, uint32_t step0,
+                       int K, int64_t B, crl_stream_t stream) {
+    if (!state) return fail(CRL_ERR_ARG, "crl_blokus_rollout: null state%s");
+    if (B < 0) return fail(CRL_ERR_ARG, "crl_blokus_rollout: negative batch%s");
+    if (K < 0) return fail(CRL_ERR_ARG, "crl_blokus_rollout: negative step count K%s");
+    if (B == 0 || K == 0) return CRL_OK;
+    CRL_LAUNCH(blokus_rollout_kernel, blocks_for(B, BLK_WARPS), 32 * BLK_WARPS, (cudaStream_t)stream, (uint4 *)state,
+               (uint2 *)result, (crl_u64 *)stats, (long long)B, (crl_u64)seed, (crl_u64)first_env, step0, K);
+    return check_launch("blokus_rollout_kernel");
+}
+
 int crl_blokus_pick(const int32_t *counts, const int32_t *action_ids, int32_t capacity, const int32_t *choice,
                     int32_t *actions, int64_t B, crl_stream_t stream) {
     if (!counts || !action_ids || !choice || !actions || capacity <= 0 || B < 0) return fail(CRL_ERR_ARG, "crl_blokus_pick: bad argument%s");

@@ -228,6 +228,15 @@ int crl_blokus_step(const void *state_in, void *state_out, const int32_t *action
 /* uniform random policy over a generated list: ids[g][philox(env, step, tag 2)[0] % counts[g]], -1 if empty */
 int crl_blokus_policy_random(const int32_t *counts, const int32_t *action_ids, int32_t capacity, int32_t *actions,
                              uint64_t seed, uint64_t first_env, uint32_t step, int64_t B, crl_stream_t stream);
+/* K fused random-policy steps with auto-reset: identical to K x (crl_blokus_legal(player -1, CRL_FLAG_AUTO_RESET)
+ * -> crl_blokus_policy_random(step0 + t) -> crl_blokus_step(CRL_FLAG_AUTO_RESET)) whenever every list fits the
+ * capacity of that sequence.  No list is materialised: the pick is ids[philox(env, step0 + t, tag 2)[0] % n] over the
+ * FULL list of length n, so the trajectories equal the oracle's (oracle_rollout.c) for any list length, and the
+ * three-launch sequence's only while counts <= its capacity (it draws from the stored prefix otherwise).
+ * result (may be NULL): the 8-byte record of the last step.  stats (may be NULL): the same slots the three launches add
+ * (CRL_ST_NVALID included), counted per game in 64 bits, so any K is accepted.  B == 0 or K == 0: no-op. */
+int crl_blokus_rollout(void *state, uint8_t *result_or_null, int64_t *stats_or_null, uint64_t seed,
+                       uint64_t first_env, uint32_t step0, int K, int64_t B, crl_stream_t stream);
 /* a host-side policy's choice (the agent of match_server.py:201-218 answers with one of the strings valid_actions gave
  * it): actions[g] = action_ids[g][choice[g]], -1 (pass) if choice[g] < 0 or >= counts[g].  The policy only needs the list
  * lengths on the host; the lists stay on the device. */
