@@ -5,8 +5,6 @@
 #ifndef CRL_HOSTSIM
 #include <cuda_runtime.h>
 #include <cuda.h>            // CUtensorMap (types only: the encoder is fetched with cudaGetDriverEntryPoint, no -lcuda)
-#define CRL_LAUNCH(kernel, grid, block, stream, ...) kernel<<<(grid), (block), 0, (stream)>>>(__VA_ARGS__)
-#define CRL_LAUNCH_SMEM(kernel, grid, block, smem, stream, ...) kernel<<<(grid), (block), (smem), (stream)>>>(__VA_ARGS__)
 // dynamic shared memory (sized at launch); the emulator gives it its maximum size statically
 #define CRL_DYN_SMEM(name, maxbytes) extern __shared__ __align__(128) uint8_t name[]
 // launch with the programmatic-stream-serialization attribute (PDL); the kernel must call pdl_wait() before it
@@ -16,24 +14,8 @@ static inline bool crl_use_pdl() {
     static const bool on = !(getenv("CRL_PDL") && atoi(getenv("CRL_PDL")) == 0);
     return on;
 }
-#define CRL_LAUNCH_PDL(kernel, grid_, block_, stream_, ...)                                         \
-    do {                                                                                          \
-        cudaLaunchConfig_t cfg_ = {};                                                             \
-        cfg_.gridDim = dim3(grid_); cfg_.blockDim = dim3(block_); cfg_.dynamicSmemBytes = 0;        \
-        cfg_.stream = (stream_);                                                                  \
-        cudaLaunchAttribute at_[1];                                                               \
-        at_[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;                           \
-        at_[0].val.programmaticStreamSerializationAllowed = 1;                                    \
-        cfg_.attrs = at_; cfg_.numAttrs = crl_use_pdl() ? 1 : 0;                                   \
-        cudaLaunchKernelEx(&cfg_, kernel, __VA_ARGS__);                                           \
-    } while (0)
 #else
 // tests/hostsim/cuda_shim.h was included first: kernels run on the SIMT emulator (CPU unit tests only)
-#define CRL_LAUNCH(kernel, grid, block, stream, ...) \
-    hostsim::launch(dim3(grid), dim3(block), [&] { kernel(__VA_ARGS__); })
-#define CRL_LAUNCH_PDL CRL_LAUNCH
-#define CRL_LAUNCH_SMEM(kernel, grid, block, smem, stream, ...) \
-    hostsim::launch(dim3(grid), dim3(block), [&] { kernel(__VA_ARGS__); })
 #define CRL_DYN_SMEM(name, maxbytes) static __attribute__((aligned(128))) uint8_t name[maxbytes]
 #endif
 
