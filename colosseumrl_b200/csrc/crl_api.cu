@@ -199,8 +199,8 @@ static int tron_place(TronShape &s, int ring_offset = 1, const int *spawn_offset
     return CRL_OK;
 }
 
-// Tensor map of the plane part of a Tron state buffer: [12 rows][B*4 uint32], row pitch B*16 bytes, box = 12 rows x
-// tile*4 words.  The driver's encoder is fetched through the runtime (no link-time dependency on libcuda); the last
+// Tensor map of the plane part of a Tron state buffer: [rows][B*4 uint32] (rows = TRON_PVEC), row pitch B*16 bytes,
+// box = rows x tile*4 words.  The driver's encoder is fetched through the runtime (no link-time dependency on libcuda); the last
 // few maps are cached per thread because an actor steps the same buffers over and over.
 #ifndef CRL_HOSTSIM
 typedef CUresult (*crl_encode_fn)(CUtensorMap *, CUtensorMapDataType, cuuint32_t, void *, const cuuint64_t *, const cuuint64_t *,
@@ -236,7 +236,7 @@ static int tron_plane_map(const void *state, int64_t B, int tile, int rows, CUte
 }
 #endif
 
-// environments (= threads) per CTA of the step / rollout kernels: 64 (13 KB of shared memory, ~7 CTAs per SM at
+// environments (= threads) per CTA of the step / rollout kernels: 64 (10 KB of shared memory, ~7 CTAs per SM at
 // B = 65,536); CRL_TRON_TILE=32 for exploration
 static int tron_tile() {
     static const int tile = [] {
@@ -453,7 +453,8 @@ int crl_tron_step_spawns(const void *state_in, void *state_out, const int8_t *ac
     TronMaps maps;
     const int tile = tron_tile();
 #ifndef CRL_HOSTSIM
-    if ((rc = tron_plane_map(state_in, B, tile, 12, &maps.in)) || (rc = tron_plane_map(state_out, B, tile, 12, &maps.out)))
+    if ((rc = tron_plane_map(state_in, B, tile, TRON_PVEC, &maps.in)) ||
+        (rc = tron_plane_map(state_out, B, tile, TRON_PVEC, &maps.out)))
         return rc;
 #else
     maps.in_ptr = (const uint4 *)state_in; maps.out_ptr = (uint4 *)state_out;

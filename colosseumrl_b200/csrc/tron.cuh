@@ -7,9 +7,13 @@
 //   TronGridEnvironment.new_state :228-263                                  (tron_reset_kernel / auto-reset)
 //   state_to_observation :363-405 + relative_player_inplace CyTronGrid.pyx:65-71 (tron_observe_kernel)
 //
-// HBM layout (SoA of 16-byte vectors, [13][B] uint4, 208 B per environment):
-//   vector v = 3*p + j (p = player plane 0..3, j = 0..2): 32-bit words 4j..4j+3 of plane p's bitboard,
-//             bit (y*N + x) of the 384-bit plane is set iff player p owns cell (x, y)   (N*N <= 384, N <= 19)
+// HBM layout (SoA of 16-byte vectors, [13][B] uint4, 208 B per environment, of which 160 B are moved by a step):
+//   A cell holds its owner code: 0 empty, q + 1 for player q.  The code is stored in binary, one 384-bit plane per bit:
+//     plane c0 = players 0 and 2 (codes 1, 3), c1 = players 1 and 2 (codes 2, 3), c2 = player 3 (code 4)
+//   vector v = 3*k + j (k = code bit-plane 0..2, j = 0..2): 32-bit words 4j..4j+3 of plane k,
+//             bit (y*N + x) of the plane is bit k of the owner code of cell (x, y)   (N*N <= 384, N <= 19)
+//   vectors 9..11 = reserved: always zero (reset, pack and an out-of-place step write zeros; the step and rollout
+//             kernels never read them), so two states holding the same game are equal byte for byte
 //   vector 12 = header, one BYTE LANE per player so that the four players are advanced with 32-bit SWAR
 //   arithmetic:
 //     .x byte p = (head x + 1) | direction << 5          (coordinates are stored biased by one: 0 and N+1 are
@@ -18,20 +22,22 @@
 //     .w = cells3 | episode steps << 9
 //
 // Data movement: vector v of the TILE environments of a CTA is ONE contiguous global segment (TILE*16 bytes), so
-// the tile travels as 13 bulk-async copies (TMA, cp.async.bulk -> SASS UBLKCP) issued by one thread into shared
-// memory and 13 back; the planes are never unpacked into registers.  Each thread owns one environment and only
-// touches the <= 16 bitboard words its players move into plus the 16-byte header.
+// the tile travels as one 2-D tensor copy of the 9 plane vectors plus one bulk copy of the header (TMA) issued by one
+// thread into shared memory, and the same two copies back; the planes are never unpacked into registers.  Each thread
+// owns one environment and only touches the <= 12 bitboard words its players move into plus the 16-byte header.
 //
 // The step is split in three phases so that only the middle one is exposed between the loads and the stores:
 //   phase 1 (header + actions have landed, planes still in flight): new directions / target cells / addresses
-//   phase 2 (planes have landed): 16 board lookups, the reference's player-order-sequential resolve, <= 4 bit sets;
-//           then the 12 plane vectors are already on their way back to HBM
+//   phase 2 (planes have landed): 12 board lookups, the reference's player-order-sequential resolve, <= 4 bit sets;
+//           then the 9 plane vectors are already on their way back to HBM
 //   phase 3 (plane stores in flight): rewards / terminal / winners / ranking / header / result record / statistics
 #pragma once
 #include "crl_common.cuh"
 #include "philox.cuh"
 
-#define TRON_VEC 13
+#define TRON_VEC 13          // 16-byte vectors per environment in a state buffer
+#define TRON_PVEC 9          // vectors 0..8: the three owner-code bit-planes
+#define TRON_HVEC 12         // vector 12: the header (9..11 reserved)
 #define TRON_WORDS 6
 #define TRON_ONES 0x01010101u
 
@@ -40,7 +46,7 @@ struct TronParams {
     uint32_t pmask;                     // 0x01 in byte p for p < P
     uint32_t rkmask;                    // ranking bits of the present players: (1 << 2P) - 1
     uint32_t start_hdr[4];              // header of new_state()
-    uint32_t spawn_word[4];             // 32-bit word (0..11) of plane p that holds player p's spawn cell
+    uint32_t spawn_word[4];             // 32-bit word (0..11) of a plane that holds player p's spawn cell
     uint32_t spawn_bit[4];              // ... and the bit inside it (0 for absent players)
 };
 
@@ -84,13 +90,15 @@ __host__ __device__ __forceinline__ uint4 tron_hdr_encode(const TronHdr &s) {
 }
 
 // ---- the shared-memory tile ---------------------------------------------------------------------------------
+// rows 0..8 = the plane vectors 0..8 of the buffer, row 9 = its header vector 12 (the reserved vectors stay in HBM)
 template <int TILE>
 struct TronTile {
-    uint4 v[TRON_VEC][TILE];
+    uint4 v[TRON_PVEC + 1][TILE];
     static constexpr int PL = 3 * TILE * 4;     // distance in 32-bit words between the same word of two planes
-    // 32-bit view of environment t: word j (0..11) of plane q is words(t)[woff(j) + q * PL]
+    // 32-bit view of environment t: word j (0..11) of plane k is words(t)[woff(j) + k * PL]
     __device__ __forceinline__ uint32_t *words(int t) { return reinterpret_cast<uint32_t *>(&v[0][t]); }
     __device__ __forceinline__ static int woff(int j) { return (j >> 2) * (TILE * 4) + (j & 3); }
+    __device__ __forceinline__ uint4 *hdr() { return &v[TRON_PVEC][0]; }
 };
 
 template <int TILE>
@@ -98,7 +106,7 @@ __device__ __forceinline__ void tron_cta_sync() {
     if (TILE == 32) __syncwarp(); else __syncthreads();
 }
 
-// Tensor maps of the [12][B*4] uint32 plane part of a state buffer (box = 12 rows x TILE*4 words): one for the
+// Tensor maps of the [9][B*4] uint32 plane part of a state buffer (box = 9 rows x TILE*4 words): one for the
 // buffer the step reads, one for the buffer it writes.  Built on the host per call (crl_api.cu).
 struct TronMaps {
 #ifndef CRL_HOSTSIM
@@ -109,8 +117,8 @@ struct TronMaps {
 #endif
 };
 
-// global -> shared, two transactions: the header vector (barrier 0, one 1-D bulk copy) and the 12 plane vectors
-// (barrier 1, one 2-D tensor copy when a map is given, else 12 bulk copies)
+// global -> shared, two transactions: the header vector (barrier 0, one 1-D bulk copy) and the 9 plane vectors
+// (barrier 1, one 2-D tensor copy when a map is given, else 9 bulk copies)
 template <int TILE>
 __device__ __forceinline__ void tron_tile_load_issue(TronTile<TILE> &tile, uint64_t *bar, const TronMaps *maps,
                                                      const uint4 *__restrict__ st, long long B, long long e0, int n) {
@@ -119,20 +127,22 @@ __device__ __forceinline__ void tron_tile_load_issue(TronTile<TILE> &tile, uint6
         mbar_init(&bar[0], 1);
         mbar_init(&bar[1], 1);
         mbar_expect_tx(&bar[0], (uint32_t)(n * 16));
-        bulk_g2s(&tile.v[12][0], st + 12ll * B + e0, (uint32_t)(n * 16), &bar[0]);
+        bulk_g2s(tile.hdr(), st + TRON_HVEC * B + e0, (uint32_t)(n * 16), &bar[0]);
         if (maps) {
-            mbar_expect_tx(&bar[1], (uint32_t)(12 * TILE * 16));             // clipped columns are zero-filled and count
+            mbar_expect_tx(&bar[1], (uint32_t)(TRON_PVEC * TILE * 16));      // clipped columns are zero-filled and count
             tma_load_2d(&tile.v[0][0], &maps->in, (int)(e0 * 4), 0, &bar[1]);
         } else {
-            mbar_expect_tx(&bar[1], (uint32_t)(12 * n * 16));
+            mbar_expect_tx(&bar[1], (uint32_t)(TRON_PVEC * n * 16));
 #pragma unroll
-            for (int v = 0; v < 12; v++) bulk_g2s(&tile.v[v][0], st + (long long)v * B + e0, (uint32_t)(n * 16), &bar[1]);
+            for (int v = 0; v < TRON_PVEC; v++) bulk_g2s(&tile.v[v][0], st + (long long)v * B + e0, (uint32_t)(n * 16), &bar[1]);
         }
     }
     tron_cta_sync<TILE>();     // barrier initialisation visible to the waiters
 #else
-    for (int v = 0; v < TRON_VEC; v++)
-        if ((int)threadIdx.x < n) tile.v[v][threadIdx.x] = st[(long long)v * B + e0 + threadIdx.x];
+    if ((int)threadIdx.x < n) {
+        for (int v = 0; v < TRON_PVEC; v++) tile.v[v][threadIdx.x] = st[(long long)v * B + e0 + threadIdx.x];
+        tile.hdr()[threadIdx.x] = st[TRON_HVEC * B + e0 + threadIdx.x];
+    }
     tron_cta_sync<TILE>();
 #endif
 }
@@ -143,7 +153,7 @@ __device__ __forceinline__ void tron_tile_wait(uint64_t *bar, int which) {
 #endif
 }
 
-// shared -> global: the 12 plane vectors (planes == true) or the header vector (the last store of the CTA)
+// shared -> global: the 9 plane vectors (planes == true) and / or the header vector (the last store of the CTA)
 template <int TILE>
 __device__ __forceinline__ void tron_tile_store(TronTile<TILE> &tile, const TronMaps *maps, uint4 *__restrict__ st,
                                                 long long B, long long e0, int n, bool planes, bool hdr) {
@@ -156,17 +166,20 @@ __device__ __forceinline__ void tron_tile_store(TronTile<TILE> &tile, const Tron
                 tma_store_2d(&maps->out, (int)(e0 * 4), 0, &tile.v[0][0]);
             } else {
 #pragma unroll
-                for (int v = 0; v < 12; v++) bulk_s2g(st + (long long)v * B + e0, &tile.v[v][0], (uint32_t)(n * 16));
+                for (int v = 0; v < TRON_PVEC; v++) bulk_s2g(st + (long long)v * B + e0, &tile.v[v][0], (uint32_t)(n * 16));
             }
         }
-        if (hdr) bulk_s2g(st + 12ll * B + e0, &tile.v[12][0], (uint32_t)(n * 16));
+        if (hdr) bulk_s2g(st + TRON_HVEC * B + e0, tile.hdr(), (uint32_t)(n * 16));
         bulk_commit();
         if (hdr) bulk_wait_read();       // the tile may be released once the copies have read it
     }
 #else
     tron_cta_sync<TILE>();
-    for (int v = planes ? 0 : 12; v < (hdr ? 13 : 12); v++)
-        if ((int)threadIdx.x < n) st[(long long)v * B + e0 + threadIdx.x] = tile.v[v][threadIdx.x];
+    if ((int)threadIdx.x < n) {
+        if (planes)
+            for (int v = 0; v < TRON_PVEC; v++) st[(long long)v * B + e0 + threadIdx.x] = tile.v[v][threadIdx.x];
+        if (hdr) st[TRON_HVEC * B + e0 + threadIdx.x] = tile.hdr()[threadIdx.x];
+    }
     tron_cta_sync<TILE>();
 #endif
 }
@@ -178,8 +191,9 @@ __device__ __forceinline__ void tron_tile_store(TronTile<TILE> &tile, const Tron
 // The four players live in the four byte lanes of 32-bit words.  Per-player flags are "byte flags" (0x01 in byte p).
 // The reference's loop is sequential in the player index, but the only things a later player can observe from an
 // earlier one in the same step are (a) the single cell it just claimed, (b) its new head and (c) a head-on kill.
-// So all lookups are done against the OLD board (16 independent shared-memory loads), the sequential part runs on
-// registers only, and the <= 4 bit sets are independent stores (plane i is written by player i alone).
+// So all lookups are done against the OLD board (12 independent shared-memory loads) and the sequential part runs on
+// registers only.  The <= 4 bit sets are read-modify-writes of the tile, in player order: players 0 and 2 share plane
+// c0, players 1 and 2 plane c1, and two movers may claim different cells of the same 32-bit word.
 struct TronCtx {
     uint32_t X, Y, Z, W;            // header words (updated in place by the phases)
     uint32_t BX, BY, NX, NY;        // biased head coordinates, old / candidate (one byte per player)
@@ -235,19 +249,21 @@ __device__ __forceinline__ void tron_phase2(TronCtx &c, TronTile<TILE> &tile, in
     uint32_t *words = tile.words(t);
     if (c.reset) {                                                        // new_state (py:228-263): empty board, p+1 at each head
 #pragma unroll
-        for (int v = 0; v < 12; v++) tile.v[v][t] = make_uint4(0u, 0u, 0u, 0u);
+        for (int v = 0; v < TRON_PVEC; v++) tile.v[v][t] = make_uint4(0u, 0u, 0u, 0u);
 #pragma unroll
-        for (int p = 0; p < 4; p++) words[TronTile<TILE>::woff((int)prm.spawn_word[p]) + p * PL] = prm.spawn_bit[p];
+        for (int p = 0; p < 4; p++)                                       // spawns may share a word: OR by code p + 1
+#pragma unroll
+            for (int k = 0; k < 3; k++)
+                if (((p + 1) >> k) & 1) words[TronTile<TILE>::woff((int)prm.spawn_word[p]) + k * PL] |= prm.spawn_bit[p];
     }
-    uint32_t own[4], HK[4], vown[4];
+    uint32_t own[4], HK[4];
 #pragma unroll
     for (int i = 0; i < 4; i++) {
         const uint32_t *wp = words + c.off[i];
-        const uint32_t v0 = wp[0], v1 = wp[PL], v2 = wp[2 * PL], v3 = wp[3 * PL];
-        vown[i] = (i == 0) ? v0 : (i == 1) ? v1 : (i == 2) ? v2 : v3;
-        const bool f0 = v0 & c.bit[i], f1 = v1 & c.bit[i], f2 = v2 & c.bit[i], f3 = v3 & c.bit[i];
-        own[i] = f3 ? 0x01000000u : f2 ? 0x00010000u : f1 ? 0x00000100u : f0 ? 0x00000001u : 0u;   // owner of the cell, byte flag
-        const uint32_t hs = f3 ? c.hpos[3] : f2 ? c.hpos[2] : f1 ? c.hpos[1] : c.hpos[0];
+        const uint32_t v0 = wp[0], v1 = wp[PL], v2 = wp[2 * PL];
+        const uint32_t code = (v0 & c.bit[i] ? 1u : 0u) | (v1 & c.bit[i] ? 2u : 0u) | (v2 & c.bit[i] ? 4u : 0u);
+        own[i] = code ? 1u << (8 * (code - 1u)) : 0u;                     // owner of the cell (code - 1), byte flag
+        const uint32_t hs = code == 4u ? c.hpos[3] : code == 3u ? c.hpos[2] : code == 2u ? c.hpos[1] : c.hpos[0];
         HK[i] = (hs == c.pos[i]) ? own[i] : 0u;                           // ... and whether the cell is that owner's (old) head
     }
     uint32_t D4 = c.D4, ALV = c.ALV, MVB = 0u, ACTB = 0u;
@@ -273,8 +289,11 @@ __device__ __forceinline__ void tron_phase2(TronCtx &c, TronTile<TILE> &tile, in
         ACTB |= act ? me : 0u;
     }
 #pragma unroll
-    for (int i = 0; i < 4; i++)
-        if (MVB & (1u << (8 * i))) words[c.off[i] + i * PL] = vown[i] | c.bit[i];
+    for (int i = 0; i < 4; i++)                                           // mover i sets its bit in the planes of code i + 1
+        if (MVB & (1u << (8 * i)))
+#pragma unroll
+            for (int k = 0; k < 3; k++)
+                if (((i + 1) >> k) & 1) words[c.off[i] + k * PL] |= c.bit[i];
     const uint32_t AM = ACTB * 3u, MM = MVB * 0x1Fu;
     const uint32_t dirn = (c.DIR & ~AM) | (c.ND & AM);                    // pyx:44 (also when i dies)
     c.X = (c.BX & ~MM) | (c.NX & MM) | dirn << 5;
@@ -396,7 +415,7 @@ tron_step_kernel(const __grid_constant__ TronMaps maps, const uint4 *__restrict_
 #ifndef CRL_HOSTSIM
     if (t == 0 && !(flags & 0x2000)) {
         l2_prefetch_tensor_2d(&maps.in, (int)(e0 * 4), 0);
-        l2_prefetch_bulk(in + 12ll * B + e0, (uint32_t)(n * 16));
+        l2_prefetch_bulk(in + TRON_HVEC * B + e0, (uint32_t)(n * 16));
         const uint32_t abytes = (uint32_t)((flags & CRL_FLAG_PACKED_ACTIONS) ? n : 4 * n);
         const char *ap = (const char *)actions + ((flags & CRL_FLAG_PACKED_ACTIONS) ? e0 : 4 * e0);
         if (!(abytes & 15u) && !((uintptr_t)ap & 15)) l2_prefetch_bulk(ap, abytes);
@@ -431,14 +450,14 @@ tron_step_kernel(const __grid_constant__ TronMaps maps, const uint4 *__restrict_
     // phase 3, 0x800 no statistics -- results are meaningless with any of them; 0x1000 late PDL trigger, 0x2000 no
     // prologue prefetch (results unaffected)
     const bool work = valid && !(flags & 0x100);
-    if (work) tron_phase1<TILE>(c, tile.v[12][t], a, prm, (flags & CRL_FLAG_AUTO_RESET) != 0);
+    if (work) tron_phase1<TILE>(c, tile.hdr()[t], a, prm, (flags & CRL_FLAG_AUTO_RESET) != 0);
     tron_tile_wait(bar, 1);
     if (work && !(flags & 0x200)) tron_phase2(c, tile, t, prm);
     tron_tile_store(tile, &maps, out, B, e0, n, true, false);
     if (flags & 0x1000) pdl_launch_dependents();     // (diagnostic: the round-1 trigger position)
     if (work) {
         if (!(flags & 0x400)) tron_phase3(c, prm, o);
-        tile.v[12][t] = tron_ctx_header(c);
+        tile.hdr()[t] = tron_ctx_header(c);
         const uint2 rec = tron_pack_result(o);
         if (flags & CRL_FLAG_COMPACT2_RESULT)                                        // 2-byte record (see the header)
             ((uint16_t *)result)[e0 + t] = (uint16_t)(((rec.y >> 8) & 0xfu) | (rec.y & 1u) << 4 | (rec.y >> 24) << 8);
@@ -446,6 +465,9 @@ tron_step_kernel(const __grid_constant__ TronMaps maps, const uint4 *__restrict_
         else result[e0 + t] = rec;
     }
     tron_tile_store(tile, &maps, out, B, e0, n, false, true);
+    if (out != in && valid)                                  // an out-of-place step writes a whole state: reserved = 0
+#pragma unroll
+        for (int v = TRON_PVEC; v < TRON_HVEC; v++) out[(long long)v * B + e0 + t] = make_uint4(0u, 0u, 0u, 0u);
     // statistics: every warp adds its 17 sums straight to the CTA's row of the global buffer (fire-and-forget RED);
     // after the last store, so that the header is already draining (measured 0.1 us / step cheaper than before it)
     if (stats && !(flags & 0x800))
@@ -475,7 +497,7 @@ tron_rollout_kernel(uint4 *__restrict__ state, uint2 *__restrict__ result, crl_u
     tron_zero_out(o);
     TronCtx c;
     c.Z = c.W = 0u;
-    uint4 h = valid ? tile.v[12][t] : make_uint4(0u, 0u, 0u, 0u);
+    uint4 h = valid ? tile.hdr()[t] : make_uint4(0u, 0u, 0u, 0u);
     for (int k = 0; k < K; k++) {
         if (valid) {
             uint4 r = env_words(seed, first_env + (crl_u64)(e0 + t), step0 + (uint32_t)k, CRL_TAG_TRON);
@@ -491,7 +513,7 @@ tron_rollout_kernel(uint4 *__restrict__ state, uint2 *__restrict__ result, crl_u
         if (stats) tron_stats<int, int>(sm_stat, valid, o, c.Z, c.W, lane_const);
     }
     if (valid) {
-        tile.v[12][t] = h;
+        tile.hdr()[t] = h;
         if (result) result[e0 + t] = tron_pack_result(o);
     }
     tron_tile_store(tile, (const TronMaps *)nullptr, state, B, e0, n, true, true);
@@ -519,25 +541,27 @@ __global__ void tron_reset_kernel(uint4 *__restrict__ state, const uint8_t *__re
     const int v = (int)(idx / B);
     const long long e = idx - (long long)v * B;
     if (mask && !mask[e]) return;
-    uint4 val = make_uint4(prm.start_hdr[0], prm.start_hdr[1], prm.start_hdr[2], prm.start_hdr[3]);
+    uint4 val = v == TRON_HVEC ? make_uint4(prm.start_hdr[0], prm.start_hdr[1], prm.start_hdr[2], prm.start_hdr[3])
+                               : make_uint4(0u, 0u, 0u, 0u);        // (reserved vectors 9..11: zero)
+    if (v < TRON_PVEC) {                                             // words 4j .. 4j+3 of plane k: the spawn bits of codes with bit k
+        const uint32_t k = (uint32_t)v / 3u, j = (uint32_t)v - 3u * k;
 #pragma unroll
-    for (int p = 0; p < 4; p++)
-#pragma unroll
-        for (int j = 0; j < 3; j++)
-            if (v == 3 * p + j) {                                        // words 4j .. 4j+3 of plane p: the spawn bit only
-                const uint32_t w = prm.spawn_word[p], b = prm.spawn_bit[p];
-                val = make_uint4(w == 4u * j ? b : 0u, w == 4u * j + 1u ? b : 0u, w == 4u * j + 2u ? b : 0u, w == 4u * j + 3u ? b : 0u);
-            }
+        for (int p = 0; p < 4; p++) {
+            const uint32_t w = prm.spawn_word[p], b = (((p + 1) >> k) & 1) ? prm.spawn_bit[p] : 0u;   // spawns may share a word
+            val.x |= w == 4u * j ? b : 0u; val.y |= w == 4u * j + 1u ? b : 0u;
+            val.z |= w == 4u * j + 2u ? b : 0u; val.w |= w == 4u * j + 3u ? b : 0u;
+        }
+    }
     state[idx] = val;
 }
 
-// state_to_observation (TronGridEnvironment.py:385-405).  A CTA handles a tile of 16 environments: 13 bulk copies
+// state_to_observation (TronGridEnvironment.py:385-405).  A CTA handles a tile of 16 environments: 10 bulk copies
 // bring their packed state into shared memory, its 4 warps unpack 4 environments each into a shared-memory image of
 // the dense output, and ONE bulk copy writes the tile's boards (16 * nview * N*N contiguous bytes, always 16-byte
 // aligned and a multiple of 16 bytes) back to HBM.
-// Unpacking is byte-SWAR: lane l owns cells 128 k + 4 l .. + 3 (k = 0..2): the 4 bits of every plane are spread to
-// 4 bytes with one multiply + mask, and the relabelled owner is sum_q plane_q * newid_q with newid_q a constant of
-// (plane q, viewer) -- the relabelling of CyTronGrid.pyx:65-71 costs nothing.
+// Unpacking is byte-SWAR: lane l owns cells 128 k + 4 l .. + 3 (k = 0..2): the 4 bits of every code plane are spread
+// to 4 bytes with one multiply + mask, which gives the owner code of each cell, and one PRMT through a per-viewer
+// table relabels it -- the relabelling of CyTronGrid.pyx:65-71 costs nothing.
 //   player >= 0 : that player's view (board relabelled, vectors rolled py:392)
 //   player == -1: absolute view (plain unpack: board values p+1)
 //   player == -3: ALL P views at once (CRL_PLAYER_ALL, nview = P)
@@ -583,17 +607,20 @@ tron_observe_kernel(const uint4 *__restrict__ st, long long B, TronParams prm, i
 #ifndef CRL_HOSTSIM
     if (threadIdx.x == 0) {
         mbar_init(&bar[0], 1);
-        mbar_expect_tx(&bar[0], (uint32_t)(TRON_VEC * n * 16));
+        mbar_expect_tx(&bar[0], (uint32_t)((TRON_PVEC + 1) * n * 16));
         const uint4 *src = st + e0;
         uint4 *dst = &tile.v[0][0];
 #pragma unroll 1
-        for (int v = 0; v < TRON_VEC; v++, src += B, dst += TRON_OBS_TILE) bulk_g2s(dst, src, (uint32_t)(n * 16), &bar[0]);
+        for (int v = 0; v < TRON_PVEC; v++, src += B, dst += TRON_OBS_TILE) bulk_g2s(dst, src, (uint32_t)(n * 16), &bar[0]);
+        bulk_g2s(tile.hdr(), st + TRON_HVEC * B + e0, (uint32_t)(n * 16), &bar[0]);
     }
     __syncthreads();
     mbar_wait(&bar[0], 0);
 #else
-    for (int v = 0; v < TRON_VEC; v++)
-        if ((int)threadIdx.x < n) tile.v[v][threadIdx.x] = st[(long long)v * B + e0 + threadIdx.x];
+    if ((int)threadIdx.x < n) {
+        for (int v = 0; v < TRON_PVEC; v++) tile.v[v][threadIdx.x] = st[(long long)v * B + e0 + threadIdx.x];
+        tile.hdr()[threadIdx.x] = st[TRON_HVEC * B + e0 + threadIdx.x];
+    }
     __syncthreads();
 #endif
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -607,10 +634,8 @@ tron_observe_kernel(const uint4 *__restrict__ st, long long B, TronParams prm, i
         const uint32_t *wp = tile.words(t) + wl;
         uint8_t *out = img + t * nview * NN + 4 * lane;
         for (int k = 0; k < chunks; k++, wp += TRON_OBS_TILE * 4, out += 128) {
-            // owner (0 empty, q + 1) of the lane's 4 cells, one byte each: the planes are disjoint, so the three BIT-PLANES of
-            // the owner value are p0 | p2, p1 | p2 and p3 -- three nibble -> bytes spreads instead of four
-            const uint32_t p0 = wp[0], p1 = wp[PL], p2 = wp[2 * PL], p3 = wp[3 * PL];
-            const uint32_t v0 = ((p0 | p2) >> sh) & 15u, v1 = ((p1 | p2) >> sh) & 15u, v2 = (p3 >> sh) & 15u;
+            // owner code (0 empty, q + 1) of the lane's 4 cells, one byte each, from the three stored code bit-planes
+            const uint32_t v0 = (wp[0] >> sh) & 15u, v1 = (wp[PL] >> sh) & 15u, v2 = (wp[2 * PL] >> sh) & 15u;
             const uint32_t ow = ((v0 * 0x00204081u) & TRON_ONES) + 2u * ((v1 * 0x00204081u) & TRON_ONES) +
                                 4u * ((v2 * 0x00204081u) & TRON_ONES);
             const uint32_t sel = __byte_perm(ow | ow >> 4, 0u, 0x4420);      // the 4 owners as PRMT selector nibbles
@@ -636,14 +661,14 @@ tron_observe_kernel(const uint4 *__restrict__ st, long long B, TronParams prm, i
             const int pv = ALL ? r / P : max(player, 0), c = ALL ? r - pv * P : r;
             int src = c + ((!ALL && player == -1) ? 0 : pv);
             src -= src >= P ? P : 0;
-            const uint4 h = tile.v[12][t];
+            const uint4 h = tile.hdr()[t];
             const uint32_t bx = (h.x >> (8 * src)) & 255u, by = (h.y >> (8 * src)) & 255u;
             const long long o = e0 * per_env + i;
             if (heads) heads[o] = ((int)(by & 31u) - 1) * N + (int)(bx & 31u) - 1;
             if (dirs) dirs[o] = (int)(bx >> 5) & 3;
             if (deaths) deaths[o] = (int)(by >> 5);
         }
-        if (terminal && (int)threadIdx.x < n) terminal[e0 + threadIdx.x] = (uint8_t)((tile.v[12][threadIdx.x].z >> 27) & 1u);
+        if (terminal && (int)threadIdx.x < n) terminal[e0 + threadIdx.x] = (uint8_t)((tile.hdr()[threadIdx.x].z >> 27) & 1u);
     }
     // the tile's boards: one bulk copy when the segment is 16-byte aligned and sized, a cooperative byte copy otherwise
     const int nbytes = n * nview * NN;
@@ -669,7 +694,7 @@ tron_observe_kernel(const uint4 *__restrict__ st, long long B, TronParams prm, i
 __global__ void tron_ranking_kernel(const uint4 *__restrict__ st, long long B, TronParams prm, uint8_t *__restrict__ ranking) {
     long long e = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (e >= B) return;
-    const uint4 h = st[12ll * B + e];
+    const uint4 h = st[TRON_HVEC * B + e];
     TronCtx c;
     c.X = h.x; c.Y = h.y; c.Z = h.z; c.W = h.w;
     c.D4 = (h.y >> 5) & 0x07070707u;
@@ -686,23 +711,24 @@ __global__ void tron_pack_kernel(uint4 *__restrict__ st, long long B, TronParams
     const int N = prm.N, P = prm.P, NN = N * N;
     long long e = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (e >= B) return;
-    uint64_t pl[4][TRON_WORDS];
+    uint64_t pl[3][TRON_WORDS];                             // the three owner-code bit-planes
     TronHdr s;
 #pragma unroll
-    for (int p = 0; p < 4; p++) {
+    for (int k = 0; k < 3; k++)
 #pragma unroll
-        for (int w = 0; w < TRON_WORDS; w++) pl[p][w] = 0;
-        s.hx[p] = s.hy[p] = s.dir[p] = s.death[p] = s.cells[p] = 0;
-    }
+        for (int w = 0; w < TRON_WORDS; w++) pl[k][w] = 0;
+#pragma unroll
+    for (int p = 0; p < 4; p++) s.hx[p] = s.hy[p] = s.dir[p] = s.death[p] = s.cells[p] = 0;
     for (int c = 0; c < NN; c++) {
-        int v = board[e * NN + c];
+        const int v = board[e * NN + c];
+        const int code = (v >= 1 && v <= 4) ? v : 0;         // owner code: player v - 1
 #pragma unroll
-        for (int p = 0; p < 4; p++) {
-            s.cells[p] += (v == p + 1);
+        for (int p = 0; p < 4; p++) s.cells[p] += (code == p + 1);
+#pragma unroll
+        for (int k = 0; k < 3; k++)
 #pragma unroll
             for (int w = 0; w < TRON_WORDS; w++)
-                pl[p][w] |= (v == p + 1 && w == (c >> 6)) ? (1ull << (c & 63)) : 0ull;
-        }
+                pl[k][w] |= (((code >> k) & 1) && w == (c >> 6)) ? (1ull << (c & 63)) : 0ull;
     }
     int alive = 0;
 #pragma unroll
@@ -718,11 +744,13 @@ __global__ void tron_pack_kernel(uint4 *__restrict__ st, long long B, TronParams
     s.terminal = alive <= 1;
     s.ep_len = 0;
 #pragma unroll
-    for (int p = 0; p < 4; p++)
+    for (int k = 0; k < 3; k++)
 #pragma unroll
         for (int j = 0; j < 3; j++) {
-            uint64_t a = pl[p][2 * j], b = pl[p][2 * j + 1];
-            st[(long long)(3 * p + j) * B + e] = make_uint4((uint32_t)a, (uint32_t)(a >> 32), (uint32_t)b, (uint32_t)(b >> 32));
+            uint64_t a = pl[k][2 * j], b = pl[k][2 * j + 1];
+            st[(long long)(3 * k + j) * B + e] = make_uint4((uint32_t)a, (uint32_t)(a >> 32), (uint32_t)b, (uint32_t)(b >> 32));
         }
-    st[(long long)12 * B + e] = tron_hdr_encode(s);
+#pragma unroll
+    for (int v = TRON_PVEC; v < TRON_HVEC; v++) st[(long long)v * B + e] = make_uint4(0u, 0u, 0u, 0u);   // reserved
+    st[(long long)TRON_HVEC * B + e] = tron_hdr_encode(s);
 }

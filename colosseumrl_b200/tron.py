@@ -34,7 +34,8 @@ def parse_tron_config(config: str):
 
 @dataclass
 class TronBatchState:
-    packed: torch.Tensor                    # int32 [13, B, 4]: SoA of 16-byte vectors, 208 B per environment
+    packed: torch.Tensor                    # int32 [13, B, 4]: SoA of 16-byte vectors, 208 B per environment: 9 owner-code
+                                            # bit-plane vectors, 3 reserved (zero), the header at 12
     #                                         (shapes beyond N <= 19, P <= 4: int32 [W, B], csrc/tron_wide.cuh)
     result: Optional[torch.Tensor] = None   # uint8 [B, 8] (wide shapes: [B, 16]) written by the step that produced this state
 

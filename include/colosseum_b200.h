@@ -87,7 +87,8 @@ int crl_host_event_wait(void *event);
  * Any shape the reference's config string can name within 5 <= N <= 64, 2 <= P <= 8 (TronGridEnvironment.py:28-58;
  * CyTronGrid.pyx:8-9 takes N and P from the array shapes).  Two state layouts, chosen by the shape alone:
  *  - N <= 19 and P <= 4 (BASELINE.json's 19x19 4-player and everything near it): the tuned path.  Packed state 208 bytes
- *    per environment, SoA [13][B] of 16-byte vectors (csrc/tron.cuh); actions int8[B][4]; result 8 bytes.  Everything
+ *    per environment, SoA [13][B] of 16-byte vectors, of which a step moves 160 (three owner-code bit-planes and the
+ *    header; vectors 9..11 are reserved and zero) (csrc/tron.cuh); actions int8[B][4]; result 8 bytes.  Everything
  *    below describes this path.
  *  - every other shape: the "wide" path (csrc/tron_wide.cuh), same entry points and semantics.  Packed state uint32
  *    [W][B], W = P * ceil(N*N/32) + 2P + 1 (crl_tron_state_bytes tells); actions int8[B][8]; result 16 bytes per
