@@ -68,6 +68,14 @@ SIGNATURES = {
     "crl_blokus_pack": (_int, [_vp, _vp, _vp, _vp, _vp, _i64, _vp]),
 }
 
+# ... and of the companion header include/colosseum_b200_tron_policy.h (device-side Tron opponents)
+TRON_POLICY_SIGNATURES = {
+    "crl_tron_policy_avoid": (_int, [_vp, _vp, _int, _int, _u64, _u64, _u32, _i64, _int, _int, _int, _int,
+                                     C.POINTER(_i32), _vp]),
+    "crl_tron_rollout_avoid": (_int, [_vp, _vp, _vp, _u64, _u64, _u32, _int, _i64, _int, _int, _int, _int, _int,
+                                      C.POINTER(_i32), _vp]),
+}
+
 
 class CrlError(RuntimeError):
     pass
@@ -75,7 +83,7 @@ class CrlError(RuntimeError):
 
 def declare(lib):
     """Attach restype/argtypes for every exported symbol; raises if one is missing."""
-    for name, (res, args) in SIGNATURES.items():
+    for name, (res, args) in list(SIGNATURES.items()) + list(TRON_POLICY_SIGNATURES.items()):
         fn = getattr(lib, name)  # AttributeError if the symbol is not exported
         fn.restype = res
         fn.argtypes = args

@@ -246,6 +246,35 @@ static int tron_tile() {
     return tile;
 }
 
+// The fused rollout of a placed shape: the random-policy kernels when avoid_mask == 0, else their avoid instantiations.
+static int tron_rollout_launch(const TronShape &s, void *state, uint8_t *result, int64_t *stats, uint64_t seed,
+                               uint64_t first_env, uint32_t step0, int K, int64_t B, int avoid_mask, int noise_q16,
+                               crl_stream_t stream) {
+    return dispatch<false, true>(avoid_mask != 0, [&](auto AVOID) {
+        if (s.wide)
+            return launch("tronw_rollout_kernel", tronw_rollout_kernel<AVOID>, {blocks_for(B, 128), 128}, stream,
+                          (uint32_t *)state, (uint4 *)result, (crl_u64 *)stats, B, s.wp, (crl_u64)seed, (crl_u64)first_env,
+                          step0, K, (uint32_t)avoid_mask, (uint32_t)noise_q16);
+        return dispatch<32, 64>(tron_tile(), [&](auto T) {
+            return launch("tron_rollout_kernel", tron_rollout_kernel<T, AVOID>, {blocks_for(B, T), T}, stream,
+                          (uint4 *)state, (uint2 *)result, (crl_u64 *)stats, B, s.prm, (crl_u64)seed, (crl_u64)first_env,
+                          step0, K, (uint32_t)avoid_mask, (uint32_t)noise_q16);
+        });
+    });
+}
+
+// The checks the two avoid-policy entry points share, after the shape and pointer checks: the seat mask, the noise
+// level, then the spawns (NULL = new_state's defaults) placed into the shape's parameters.
+static int tron_avoid_args(const char *fn, TronShape &s, int seat_mask, int noise_q16, int ring_offset,
+                           const int32_t *spawn_offsets) {
+    if (seat_mask < 0 || (seat_mask >> s.wp.P) != 0) return fail(CRL_ERR_ARG, "%s: seat mask bits must be below P", fn);
+    if (noise_q16 < 0 || noise_q16 > 65536) return fail(CRL_ERR_ARG, "%s: noise_q16 must satisfy 0 <= noise_q16 <= 65536", fn);
+    int so[TRONW_MAXP];
+    if (!spawn_offsets) return tron_place(s, ring_offset);
+    tron_spawn_array(s.wp.P, spawn_offsets, so);
+    return tron_place(s, ring_offset, so);
+}
+
 /* ------------------------------------------------------------------------------------------- Tic Tac Toe helpers */
 
 // Line directions and start masks from the board dimensions (2p 3x3, 3p 3x5, 4p 3x3x3).
@@ -495,13 +524,7 @@ int crl_tron_rollout(void *state, uint8_t *result, int64_t *stats, uint64_t seed
     if (!state || K < 0) return fail(CRL_ERR_ARG, "crl_tron_rollout: bad argument");
     if ((rc = tron_place(s))) return rc;
     if (B == 0 || K == 0) return CRL_OK;
-    if (s.wide)
-        return launch("tronw_rollout_kernel", tronw_rollout_kernel, {blocks_for(B, 128), 128}, stream, (uint32_t *)state,
-                      (uint4 *)result, (crl_u64 *)stats, B, s.wp, (crl_u64)seed, (crl_u64)first_env, step0, K);
-    return dispatch<32, 64>(tron_tile(), [&](auto T) {
-        return launch("tron_rollout_kernel", tron_rollout_kernel<T>, {blocks_for(B, T), T}, stream, (uint4 *)state,
-                      (uint2 *)result, (crl_u64 *)stats, B, s.prm, (crl_u64)seed, (crl_u64)first_env, step0, K);
-    });
+    return tron_rollout_launch(s, state, result, stats, seed, first_env, step0, K, B, 0, 0, stream);
 }
 
 int crl_tron_observe(const void *state, int player, int8_t *board, int32_t *heads, int32_t *directions,
@@ -743,6 +766,44 @@ int crl_blokus_pack(void *state, const int8_t *board, const uint8_t *pieces, con
     if (B == 0) return CRL_OK;
     return launch("blokus_pack_kernel", blokus_pack_kernel, {blocks_for(B * BLK_WORDS, 256), 256}, stream, (uint4 *)state,
                   B, board, pieces, score, meta);
+}
+
+/* ------------------------------------------------------------------------------------------- Tron opponents */
+
+int crl_tron_policy_avoid(const void *state, int8_t *actions, int seat_mask, int noise_q16, uint64_t seed,
+                          uint64_t first_env, uint32_t step, int64_t B, int N, int P, int flags, int ring_offset,
+                          const int32_t *spawn_offsets, crl_stream_t stream) {
+    TronShape s;
+    int rc = tron_shape(N, P, B, s);
+    if (rc) return rc;
+    if (!state || !actions) return fail(CRL_ERR_ARG, "crl_tron_policy_avoid: null pointer");
+    if ((rc = tron_avoid_args("crl_tron_policy_avoid", s, seat_mask, noise_q16, ring_offset, spawn_offsets))) return rc;
+    if (B == 0) return CRL_OK;
+    if (s.wide) {
+        if ((uintptr_t)actions & 7) return fail(CRL_ERR_ARG, "crl_tron_policy_avoid: actions must be 8-byte aligned for wide shapes");
+        return launch("tronw_policy_avoid_kernel", tronw_policy_avoid_kernel, {blocks_for(B, 128), 128}, stream,
+                      (const uint32_t *)state, actions, B, s.wp, (uint32_t)seat_mask, (uint32_t)noise_q16, (crl_u64)seed,
+                      (crl_u64)first_env, step, flags);
+    }
+    if ((uintptr_t)state & 15) return fail(CRL_ERR_ARG, "crl_tron_policy_avoid: state must be 16-byte aligned");
+    if ((uintptr_t)actions & 3) return fail(CRL_ERR_ARG, "crl_tron_policy_avoid: actions must be 4-byte aligned");
+    return launch("tron_policy_avoid_kernel", tron_policy_avoid_kernel<64>, {blocks_for(B, 64), 64}, stream,
+                  (const uint4 *)state, (uint32_t *)actions, B, s.prm, (uint32_t)seat_mask, (uint32_t)noise_q16,
+                  (crl_u64)seed, (crl_u64)first_env, step, flags);
+}
+
+int crl_tron_rollout_avoid(void *state, uint8_t *result, int64_t *stats, uint64_t seed, uint64_t first_env,
+                           uint32_t step0, int K, int64_t B, int N, int P, int avoid_mask, int noise_q16, int ring_offset,
+                           const int32_t *spawn_offsets, crl_stream_t stream) {
+    TronShape s;
+    int rc = tron_shape(N, P, B, s);
+    if (rc) return rc;
+    if (!state) return fail(CRL_ERR_ARG, "crl_tron_rollout_avoid: null state");
+    if (K < 0) return fail(CRL_ERR_ARG, "crl_tron_rollout_avoid: negative step count K");
+    if ((rc = tron_avoid_args("crl_tron_rollout_avoid", s, avoid_mask, noise_q16, ring_offset, spawn_offsets))) return rc;
+    if (B == 0 || K == 0) return CRL_OK;
+    if (!s.wide && ((uintptr_t)state & 15)) return fail(CRL_ERR_ARG, "crl_tron_rollout_avoid: state must be 16-byte aligned");
+    return tron_rollout_launch(s, state, result, stats, seed, first_env, step0, K, B, avoid_mask, noise_q16, stream);
 }
 
 }  // extern "C"

@@ -242,20 +242,26 @@ __device__ __forceinline__ void tron_phase1(TronCtx &c, uint4 h, uint32_t a4, co
     }
 }
 
+// new_state (py:228-263) in row t of the tile: empty board, code p + 1 at each spawn
+template <int TILE>
+__device__ __forceinline__ void tron_tile_reset(TronTile<TILE> &tile, int t, const TronParams &prm) {
+    constexpr int PL = TronTile<TILE>::PL;
+    uint32_t *words = tile.words(t);
+#pragma unroll
+    for (int v = 0; v < TRON_PVEC; v++) tile.v[v][t] = make_uint4(0u, 0u, 0u, 0u);
+#pragma unroll
+    for (int p = 0; p < 4; p++)                                           // spawns may share a word: OR by code p + 1
+#pragma unroll
+        for (int k = 0; k < 3; k++)
+            if (((p + 1) >> k) & 1) words[TronTile<TILE>::woff((int)prm.spawn_word[p]) + k * PL] |= prm.spawn_bit[p];
+}
+
 // phase 2: lookups, sequential resolve, bit sets, header words X / Y / Z(cells) / W
 template <int TILE>
 __device__ __forceinline__ void tron_phase2(TronCtx &c, TronTile<TILE> &tile, int t, const TronParams &prm) {
     constexpr int PL = TronTile<TILE>::PL;
     uint32_t *words = tile.words(t);
-    if (c.reset) {                                                        // new_state (py:228-263): empty board, p+1 at each head
-#pragma unroll
-        for (int v = 0; v < TRON_PVEC; v++) tile.v[v][t] = make_uint4(0u, 0u, 0u, 0u);
-#pragma unroll
-        for (int p = 0; p < 4; p++)                                       // spawns may share a word: OR by code p + 1
-#pragma unroll
-            for (int k = 0; k < 3; k++)
-                if (((p + 1) >> k) & 1) words[TronTile<TILE>::woff((int)prm.spawn_word[p]) + k * PL] |= prm.spawn_bit[p];
-    }
+    if (c.reset) tron_tile_reset(tile, t, prm);
     uint32_t own[4], HK[4];
 #pragma unroll
     for (int i = 0; i < 4; i++) {
@@ -474,13 +480,97 @@ tron_step_kernel(const __grid_constant__ TronMaps maps, const uint4 *__restrict_
         tron_stats<crl_u64, crl_u64>(stats + (blockIdx.x & (CRL_STAT_ROWS - 1)) * CRL_NSTAT, valid, o, c.Z, c.W, lane_const);
 }
 
+// ---- the avoid policy --------------------------------------------------------------------------------------------
+// A heuristic opponent in the shape of the reference's SimpleAvoidAgent (envs/tron/rllib.py:69-96, which asks
+// env.next_cell at :85 and :91): go forward if that cell is free, else try one side, else take the other.  The
+// reference's source is not part of this repository, so the exact rule below -- the coin, the noise, the order -- is
+// THIS ENGINE'S DEFINITION, pinned by the C oracle (tests/oracle_tron_avoid.c) the way the random policy is.  For
+// seat p of environment env at step t, on the state BEFORE the step:
+//   w = philox(seed, env, t, CRL_TAG_TRON_AVOID + (p >> 2))[p & 3]
+//   (w >> 16) < noise_q16 (0..65536)  ->  {0, +1, -1}[(w & 0xFFFF) % 3]
+//   else forward if its cell is free (on the board and owner code 0; heads are owned cells),
+//   else side s = (w & 1) ? +1 (right) : -1 (left) if its cell is free, else -s.
+// `occupied(cell)` is the layout's board lookup, (hx, hy) the head, dir its direction (0 N, 1 E, 2 S, 3 W).
+template <class Occupied>
+__device__ __forceinline__ int tron_avoid_decide(int hx, int hy, int dir, int N, uint32_t w, uint32_t noise_q16,
+                                                 const Occupied &occupied) {
+    if ((w >> 16) < noise_q16) {
+        const uint32_t m = (w & 0xFFFFu) % 3u;
+        return m == 2u ? -1 : (int)m;
+    }
+    auto is_free = [&](int a) {                                           // pyx:31-41: turn, then one cell ahead
+        const int d = (dir + a) & 3;
+        const int x = hx + (d == 1) - (d == 3), y = hy + (d == 2) - (d == 0);
+        return x >= 0 && x < N && y >= 0 && y < N && !occupied(y * N + x);
+    };
+    if (is_free(0)) return 0;
+    const int side = (w & 1u) ? 1 : -1;
+    return is_free(side) ? side : -side;
+}
+
+// The avoid actions of the seats in `mask` written into the action word `a` (byte p = seat p; the other bytes are
+// kept), decided on tile row t with header h (both already reset if the game restarts in this step).  Dead seats get 0.
+// Per live seat: the three code planes of <= 3 cells, i.e. up to 9 shared-memory lookups.
+template <int TILE>
+__device__ __forceinline__ uint32_t tron_avoid_word(TronTile<TILE> &tile, int t, uint4 h, uint32_t a, const TronParams &prm,
+                                                    uint32_t mask, uint32_t noise_q16, crl_u64 seed, crl_u64 env,
+                                                    uint32_t step) {
+    constexpr int PL = TronTile<TILE>::PL;
+    const uint32_t *words = tile.words(t);
+    auto occupied = [&](int cell) {
+        const int o = TronTile<TILE>::woff(cell >> 5);
+        return (((words[o] | words[o + PL] | words[o + 2 * PL]) >> (cell & 31)) & 1u) != 0u;
+    };
+    const uint4 r = env_words(seed, env, step, CRL_TAG_TRON_AVOID);
+    const uint32_t rr[4] = {r.x, r.y, r.z, r.w};
+#pragma unroll
+    for (int p = 0; p < 4; p++) {
+        if (!((mask >> p) & 1u)) continue;
+        const uint32_t bx = (h.x >> (8 * p)) & 255u, by = (h.y >> (8 * p)) & 255u;
+        const int act = (by >> 5) ? 0 : tron_avoid_decide((int)(bx & 31u) - 1, (int)(by & 31u) - 1, (int)(bx >> 5) & 3,
+                                                          prm.N, rr[p], noise_q16, occupied);
+        a = (a & ~(0xFFu << (8 * p))) | ((uint32_t)act & 0xFFu) << (8 * p);
+    }
+    return a;
+}
+
+// crl_tron_policy_avoid: one thread per environment, actions int8[B][4] read-modify-written as one 32-bit word.  The
+// tile's 9 plane rows are loaded whole (bulk copies, 144 coalesced bytes per environment) rather than only the words
+// the lookups touch: those are up to 36 scattered 4-byte reads per environment, each costing a whole 32-byte sector,
+// and the whole rows in shared memory let the lookups be plain indexed loads.
+template <int TILE>
+__global__ void __launch_bounds__(TILE)
+tron_policy_avoid_kernel(const uint4 *__restrict__ st, uint32_t *__restrict__ actions, long long B, TronParams prm,
+                         uint32_t mask, uint32_t noise_q16, crl_u64 seed, crl_u64 first_env, uint32_t step, int flags) {
+    __shared__ __align__(128) TronTile<TILE> tile;
+    __shared__ __align__(8) uint64_t bar[2];
+    const int t = threadIdx.x;
+    const long long e0 = (long long)blockIdx.x * TILE;
+    const int n = (int)min((long long)TILE, B - e0);
+    tron_tile_load_issue(tile, bar, (const TronMaps *)nullptr, st, B, e0, n);
+    const uint32_t a = t < n ? actions[e0 + t] : 0u;                      // in flight together with the tile
+    tron_tile_wait(bar, 0);
+    tron_tile_wait(bar, 1);
+    if (t >= n) return;
+    uint4 h = tile.hdr()[t];
+    if ((flags & CRL_FLAG_AUTO_RESET) && ((h.z >> 27) & 1u)) {           // decide on the game the step will restart
+        tron_tile_reset(tile, t, prm);
+        h = make_uint4(prm.start_hdr[0], prm.start_hdr[1], prm.start_hdr[2], prm.start_hdr[3]);
+    }
+    actions[e0 + t] = tron_avoid_word(tile, t, h, a, prm, mask, noise_q16, seed, first_env + (crl_u64)(e0 + t), step);
+}
+
 // K fused steps with the in-kernel Philox random policy (action of player p = {0,+1,-1}[r_p % 3]); the tile
 // stays in shared memory between steps.  Benchmark / self-play helper; semantics identical to K tron_step calls
 // with CRL_FLAG_AUTO_RESET.
-template <int TILE>
+// AVOID: the seats of avoid_mask play the avoid policy instead (= K x policy_random -> policy_avoid(avoid_mask,
+// CRL_FLAG_AUTO_RESET) -> step(CRL_FLAG_AUTO_RESET)).  The policy reads the board the step will move on, so a finished
+// game is restarted here, before the policy, and phase 1 / 2 are told not to restart it again.
+template <int TILE, bool AVOID = false>
 __global__ void __launch_bounds__(TILE)
 tron_rollout_kernel(uint4 *__restrict__ state, uint2 *__restrict__ result, crl_u64 *stats, long long B,
-                    TronParams prm, crl_u64 seed, crl_u64 first_env, uint32_t step0, int K) {
+                    TronParams prm, crl_u64 seed, crl_u64 first_env, uint32_t step0, int K, uint32_t avoid_mask,
+                    uint32_t noise_q16) {
     __shared__ __align__(128) TronTile<TILE> tile;
     __shared__ __align__(8) uint64_t bar[2];
     __shared__ int sm_stat[CRL_NSTAT];
@@ -505,7 +595,15 @@ tron_rollout_kernel(uint4 *__restrict__ state, uint2 *__restrict__ result, crl_u
             uint32_t a = 0;
 #pragma unroll
             for (int p = 0; p < 4; p++) { const uint32_t m = rr[p] % 3u; a |= ((m == 2u) ? 0xffu : m) << (8 * p); }
-            tron_phase1<TILE>(c, h, a, prm, true);
+            if constexpr (AVOID) {
+                if ((h.z >> 27) & 1u) {
+                    tron_tile_reset(tile, t, prm);
+                    h = make_uint4(prm.start_hdr[0], prm.start_hdr[1], prm.start_hdr[2], prm.start_hdr[3]);
+                }
+                a = tron_avoid_word(tile, t, h, a, prm, avoid_mask, noise_q16, seed, first_env + (crl_u64)(e0 + t),
+                                    step0 + (uint32_t)k);
+            }
+            tron_phase1<TILE>(c, h, a, prm, !AVOID);
             tron_phase2(c, tile, t, prm);
             tron_phase3(c, prm, o);
             h = tron_ctx_header(c);

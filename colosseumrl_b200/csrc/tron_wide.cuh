@@ -21,6 +21,7 @@
 #pragma once
 #include "crl_common.cuh"
 #include "philox.cuh"
+#include "tron.cuh"             // tron_avoid_decide
 
 #define TRONW_MAXP 8
 
@@ -300,10 +301,68 @@ __global__ void tronw_policy_random_kernel(int8_t *__restrict__ actions, long lo
     *(uint2 *)(actions + e * TRONW_MAXP) = make_uint2(lo, hi);
 }
 
-// K random-policy steps with auto-reset, in place
+// The avoid policy (tron.cuh: tron_avoid_decide) for the seats in `mask`, written into act[]; the other seats keep
+// theirs, dead seats get 0.  A cell is occupied if its bit is set in any of the P player planes of `st` or, when
+// `fresh` (a game the step will restart), if it is one of new_state's spawns.  Seats 0..3 draw their word from tag
+// CRL_TAG_TRON_AVOID, seats 4..7 from the next tag.
+__device__ __forceinline__ void tronw_avoid_actions(int8_t *act, const TronWideEnv &s, const TronWideRef &st, bool fresh,
+                                                    const TronWideParams &prm, uint32_t mask, uint32_t noise_q16,
+                                                    crl_u64 seed, crl_u64 env, uint32_t step) {
+    auto occupied = [&](int cell) {
+        if (fresh) {
+            bool spawn = false;
+#pragma unroll
+            for (int q = 0; q < TRONW_MAXP; q++) spawn |= q < prm.P && prm.start_head[q] == cell;
+            return spawn;
+        }
+        uint32_t any = 0;
+#pragma unroll 1
+        for (int q = 0; q < prm.P; q++) any |= st[q * prm.WPP + (cell >> 5)];
+        return ((any >> (cell & 31)) & 1u) != 0u;
+    };
+    uint4 lo = make_uint4(0u, 0u, 0u, 0u), hi = lo;
+    if (mask & 0x0Fu) lo = env_words(seed, env, step, CRL_TAG_TRON_AVOID);
+    if (mask & 0xF0u) hi = env_words(seed, env, step, CRL_TAG_TRON_AVOID + 1u);
+    const uint32_t rr[TRONW_MAXP] = {lo.x, lo.y, lo.z, lo.w, hi.x, hi.y, hi.z, hi.w};
+#pragma unroll
+    for (int p = 0; p < TRONW_MAXP; p++)
+        if ((mask >> p) & 1u)
+            act[p] = (int8_t)(s.death[p] ? 0 : tron_avoid_decide(s.hx[p], s.hy[p], s.dir[p], prm.N, rr[p], noise_q16, occupied));
+}
+
+// crl_tron_policy_avoid on the wide layout: one thread per environment, actions int8[B][8] read-modify-written as one
+// 8-byte word.  Only the words of the <= 3 candidate cells are read, from each of the P planes: the wide layout is
+// word-major, so a warp's loads of one word index are coalesced, and the board (up to 1 KB per environment) is far
+// larger than what the lookups touch.
+__global__ void __launch_bounds__(128)
+tronw_policy_avoid_kernel(const uint32_t *__restrict__ st, int8_t *__restrict__ actions, long long B, TronWideParams prm,
+                          uint32_t mask, uint32_t noise_q16, crl_u64 seed, crl_u64 first_env, uint32_t step, int flags) {
+    const long long e = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (e >= B) return;
+    const TronWideRef src{const_cast<uint32_t *>(st) + e, B};
+    TronWideEnv s;
+    tronw_hdr_load(s, src, prm);
+    const bool fresh = (flags & CRL_FLAG_AUTO_RESET) && s.terminal;       // decide on the game the step will restart
+    if (fresh) tronw_new_hdr(s, prm);
+    uint2 a8 = *(const uint2 *)(actions + e * TRONW_MAXP);
+    int8_t act[TRONW_MAXP];
+#pragma unroll
+    for (int p = 0; p < TRONW_MAXP; p++) act[p] = (int8_t)((p < 4 ? a8.x : a8.y) >> (8 * (p & 3)));
+    tronw_avoid_actions(act, s, src, fresh, prm, mask, noise_q16, seed, first_env + (crl_u64)e, step);
+    a8 = make_uint2(0u, 0u);
+#pragma unroll
+    for (int p = 0; p < TRONW_MAXP; p++) (p < 4 ? a8.x : a8.y) |= ((uint32_t)act[p] & 255u) << (8 * (p & 3));
+    *(uint2 *)(actions + e * TRONW_MAXP) = a8;
+}
+
+// K random-policy steps with auto-reset, in place.  AVOID: the seats of avoid_mask play the avoid policy instead
+// (= K x policy_random_wide -> policy_avoid(avoid_mask, CRL_FLAG_AUTO_RESET) -> step(CRL_FLAG_AUTO_RESET)); a finished
+// game is already restarted before the actions are drawn, so the policy sees the board the step moves on.
+template <bool AVOID = false>
 __global__ void __launch_bounds__(128)
 tronw_rollout_kernel(uint32_t *__restrict__ state, uint4 *__restrict__ result, crl_u64 *stats, long long B,
-                     TronWideParams prm, crl_u64 seed, crl_u64 first_env, uint32_t step0, int K) {
+                     TronWideParams prm, crl_u64 seed, crl_u64 first_env, uint32_t step0, int K, uint32_t avoid_mask,
+                     uint32_t noise_q16) {
     __shared__ int sm_stat[CRL_NSTAT];
     BlockStats bs{sm_stat};
     if (stats) bs.init();
@@ -323,6 +382,9 @@ tronw_rollout_kernel(uint32_t *__restrict__ state, uint4 *__restrict__ result, c
             }
             int8_t act[TRONW_MAXP];
             tronw_random_actions(act, seed, first_env + (crl_u64)e, step0 + (uint32_t)k);
+            if constexpr (AVOID)
+                tronw_avoid_actions(act, s, st, false, prm, avoid_mask, noise_q16, seed, first_env + (crl_u64)e,
+                                    step0 + (uint32_t)k);
             tronw_step_env(s, st, act, prm, o);
             o.rank = tronw_ranking(s, prm);
         }

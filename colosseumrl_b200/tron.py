@@ -296,11 +296,50 @@ class BatchedTronGridEnvironment(BatchedBaseEnvironment):
         self._check(fn(out.data_ptr(), self.seed, self.first_env_id, int(step), self.batch, self._stream))
         return out
 
-    def rollout(self, state: TronBatchState, step0: int, K: int) -> TronBatchState:
-        """K random-policy steps with auto-reset in one launch (state updated in place)."""
+    def _seat_mask(self, seats) -> int:
+        """None = every seat; an int is a bit mask (bit p = seat p); otherwise an iterable of seat indices."""
+        if seats is None:
+            return (1 << self.num_players) - 1
+        if isinstance(seats, int):
+            return seats
+        mask = 0
+        for p in seats:
+            mask |= 1 << int(p)
+        return mask
+
+    def avoid_actions(self, state: TronBatchState, step: int, seats=None, noise: float = 0.0,
+                      out: Optional[torch.Tensor] = None) -> torch.Tensor:
+        """The avoid policy (include/colosseum_b200_tron_policy.h: forward if free, else a Philox coin picks the side
+        tried first) for `seats` (None = all) on the device, decided on `state` before the step.  noise: the probability
+        of a uniform random move instead.  Into `out` (int8 [B, action_stride]; new and zeroed if None): the other
+        seats' entries are left as they are, so a learner's actions can be written there first.  The spawns of the last
+        new_state() and this environment's auto_reset are used: with auto_reset, a finished game is decided on the
+        fresh game the step will restart."""
+        out = out if out is not None else torch.zeros((self.batch, self.action_stride), dtype=torch.int8,
+                                                      device=self.device)
+        if out.shape != (self.batch, self.action_stride) or out.dtype != torch.int8 or not out.is_contiguous():
+            raise ValueError("out must be a contiguous int8 tensor of shape [B, %d]" % self.action_stride)
+        self._check(self._lib.crl_tron_policy_avoid(
+            state.packed.data_ptr(), out.data_ptr(), self._seat_mask(seats), int(round(noise * 65536)), self.seed,
+            self.first_env_id, int(step), self.batch, self.N, self.num_players, self.flags & _lib.FLAG_AUTO_RESET,
+            self._ring_offset, self._spawn_offsets, self._stream))
+        return out
+
+    def rollout(self, state: TronBatchState, step0: int, K: int, avoid_seats=0, noise: float = 0.0) -> TronBatchState:
+        """K steps with auto-reset in one launch (state updated in place): every seat on the random policy, or with
+        avoid_seats (a bit mask or a list of seats) those seats on the avoid policy (`avoid_actions`, with `noise`).  The
+        random-only form restarts finished games from new_state's default spawns; the avoid form from the spawns of the
+        last new_state()."""
         if state.result is None:
             state.result = self._new_result((self.batch, self.result_bytes))
-        self._check(self._lib.crl_tron_rollout(state.packed.data_ptr(), state.result.data_ptr(), self._stats_ptr,
-                                               self.seed, self.first_env_id, int(step0), int(K), self.batch, self.N,
-                                               self.num_players, self._stream))
+        mask = self._seat_mask(avoid_seats)
+        if mask == 0 and noise == 0.0:
+            self._check(self._lib.crl_tron_rollout(state.packed.data_ptr(), state.result.data_ptr(), self._stats_ptr,
+                                                   self.seed, self.first_env_id, int(step0), int(K), self.batch, self.N,
+                                                   self.num_players, self._stream))
+            return state
+        self._check(self._lib.crl_tron_rollout_avoid(
+            state.packed.data_ptr(), state.result.data_ptr(), self._stats_ptr, self.seed, self.first_env_id, int(step0),
+            int(K), self.batch, self.N, self.num_players, mask, int(round(noise * 65536)), self._ring_offset,
+            self._spawn_offsets, self._stream))
         return state

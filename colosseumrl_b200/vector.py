@@ -63,3 +63,57 @@ class VectorEnv:
         if not self.simultaneous:                                     # players = 1 << next mover
             info["mover"] = (players >> 1) - (players >> 3)           # 1, 2, 4, 8 -> 0, 1, 2, 3
         return self._observe(), rewards, terminal, info
+
+
+class SingleAgentVectorEnv:
+    """One learner against avoid-policy opponents on the device: the batched analogue of the reference's single-player
+    Tron trainer (TronRaySinglePlayerEnvironment, envs/tron/rllib.py:119-150, whose opponents are SimpleAvoidAgent,
+    :69-96).  Every other seat plays the avoid policy of BatchedTronGridEnvironment.avoid_actions, so a step is two
+    launches (policy, step) plus the observation, and no game leaves the device:
+
+        venv = SingleAgentVectorEnv(BatchedTronGridEnvironment("", batch=4096), seat=0, noise=0.0)
+        obs = venv.reset()                           # the learner's view: {"board": [B, N, N], "heads": [B, P], ...}
+        obs, reward, done, info = venv.step(actions)  # actions int8 [B]; reward int8 [B]; done uint8 [B]
+
+    End of an episode (this engine's choice: the reference's exact single-player semantics are not available to check
+    against): `done` is set when the game is terminal OR the learner has died, since the learner's episode is over as
+    soon as it can no longer act.  Such games are restarted inside that step() call, as VectorEnv does with auto_reset,
+    so the observation returned is already the fresh game.  The opponents' Philox step is a counter kept here (reset()
+    sets it to 0); restarted games use the spawns of the environment's last new_state()."""
+
+    def __init__(self, env, seat: int = 0, noise: float = 0.0):
+        if not hasattr(env, "avoid_actions"):
+            raise TypeError("SingleAgentVectorEnv needs a Tron environment (BatchedTronGridEnvironment)")
+        if not 0 <= seat < env.num_players:
+            raise ValueError("seat must be in [0, %d)" % env.num_players)
+        self.env, self.seat, self.noise = env, int(seat), float(noise)
+        self.opponents = [p for p in range(env.num_players) if p != self.seat]
+        self.state, self.t = None, 0
+        self._actions = torch.zeros((env.batch, env.action_stride), dtype=torch.int8, device=env.device)
+
+    @property
+    def num_envs(self) -> int:
+        return self.env.batch
+
+    def _observe(self) -> Dict[str, torch.Tensor]:
+        return self.env.state_to_observation(self.state, self.seat)
+
+    def reset(self) -> Dict[str, torch.Tensor]:
+        self.state, _ = self.env.new_state()
+        self.t = 0
+        return self._observe()
+
+    def step(self, actions):
+        """actions: int8 [B], the learner's.  Returns (the learner's observation, its reward int8 [B], done uint8 [B],
+        info = {"players": alive mask, "winners": winners mask, "terminal": uint8 [B]} of the step just taken)."""
+        self._actions[:, self.seat] = self.env._dev(actions, torch.int8)
+        self.env.avoid_actions(self.state, self.t, seats=self.opponents, noise=self.noise, out=self._actions)
+        self.t += 1
+        new, players, rewards, terminal, winners = self.env.next_state(self.state, None, self._actions, out=self.state)
+        self.state = new
+        reward = rewards[:, self.seat].clone()
+        learner_dead = ((players >> self.seat) & 1) == 0
+        done = (terminal.bool() | learner_dead).to(torch.uint8)
+        info = {"players": players.clone(), "winners": winners.clone(), "terminal": terminal.clone()}
+        self.env.reset_where(self.state, done)
+        return self._observe(), reward, done, info

@@ -255,4 +255,7 @@ int crl_blokus_pack(void *state, const int8_t *board, const uint8_t *pieces, con
 #ifdef __cplusplus
 }
 #endif
+
+/* device-side Tron opponents (the avoid policy and its fused rollout) */
+#include "colosseum_b200_tron_policy.h"
 #endif
