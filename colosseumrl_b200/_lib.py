@@ -76,6 +76,12 @@ TRON_POLICY_SIGNATURES = {
                                       C.POINTER(_i32), _vp]),
 }
 
+# ... and of the companion header include/colosseum_b200_learner.h (one learner against device-side random opponents)
+LEARNER_SIGNATURES = {
+    "crl_ttt_advance": (_int, [_vp, _vp, _int, _vp, _vp, _vp, _u64, _u64, _u32, _i64, _int, _vp]),
+    "crl_blokus_advance": (_int, [_vp, _vp, _int, _vp, _vp, _u64, _u64, _u32, _i64, _vp]),
+}
+
 
 class CrlError(RuntimeError):
     pass
@@ -83,7 +89,7 @@ class CrlError(RuntimeError):
 
 def declare(lib):
     """Attach restype/argtypes for every exported symbol; raises if one is missing."""
-    for name, (res, args) in list(SIGNATURES.items()) + list(TRON_POLICY_SIGNATURES.items()):
+    for name, (res, args) in list(SIGNATURES.items()) + list(TRON_POLICY_SIGNATURES.items()) + list(LEARNER_SIGNATURES.items()):
         fn = getattr(lib, name)  # AttributeError if the symbol is not exported
         fn.restype = res
         fn.argtypes = args

@@ -212,6 +212,21 @@ class BatchedBlokusEnvironment(BatchedBaseEnvironment):
                                                  self._stream))
         return state
 
+    def advance(self, state: BlokusBatchState, actions, seat: int, step: int) -> torch.Tensor:
+        """One learner move against uniform random opponents, in place (crl_blokus_advance; the rule is stated in
+        include/colosseum_b200_learner.h): the learner at `seat` plays `actions` (int32 [B] ids, -1 = pass; None: it
+        does not move), then the other seats play until `seat` is to move again, restarting finished games.  Returns
+        the record uint8 [B, 8]: int8 learner reward (its index in the stable ascending sort of the final scores) |
+        flags (1 a game finished, 2 illegal, 4 placed, 8 the learner did not move) | winners mask | opponent moves |
+        the finished game's scores of seats 0..3."""
+        a = None if actions is None else self._dev(actions, torch.int32)
+        rec = self._new_result((self.batch, 8))
+        self._check(self._lib.crl_blokus_advance(state.packed.data_ptr(), None if a is None else a.data_ptr(), int(seat),
+                                                 rec.data_ptr(), self._stats_ptr, self.seed, self.first_env_id, int(step),
+                                                 self.batch, self._stream))
+        state.result = None
+        return rec
+
     def random_actions(self, valid, step: int, out: Optional[torch.Tensor] = None) -> torch.Tensor:
         counts, ids = valid
         out = out if out is not None else torch.empty((self.batch,), dtype=torch.int32, device=self.device)

@@ -676,6 +676,38 @@ __global__ void blokus_policy_random_kernel(const int32_t *__restrict__ counts, 
     actions[g] = n > 0 ? ids[g * cap + (long long)(r.x % (uint32_t)n)] : -1;
 }
 
+// One uniform random move of the mover of the game in sm.st (not terminal): unless the mover is known to be stuck
+// (w[87]), blk_enumerate<BLK_SELECT> counts its ids and finds the one at index r % n of the FULL list, r = word `word`
+// of philox(seed, env, step, tag); blk_step_apply applies it (a pass if n == 0).  n = the valid-move count.
+__device__ __forceinline__ BlkStepOut blk_random_move(BlkSmem &sm, crl_u64 seed, crl_u64 env, uint32_t step, uint32_t tag,
+                                                      int word, int lane, bool &zeroed, int &n) {
+    const uint32_t meta = sm.st[85];
+    const int c = (int)(meta >> 8 & 3u);
+    int aid = -1;
+    n = 0;
+    if (!(sm.st[87] >> c & 1u)) {                            // not known to be stuck (w[87]): enumerate
+        const uint4 w = env_words(seed, env, step, tag);
+        const uint32_t r = word == 0 ? w.x : word == 1 ? w.y : word == 2 ? w.z : w.w;
+        n = blk_enumerate<BLK_SELECT>(sm, c, (int)(meta & 0xffu), sm.st[80 + c], lane, nullptr, 0, r, &aid);
+    }
+    return blk_step_apply(sm, aid, lane, zeroed);
+}
+
+// Statistics slot `lane` of one env-step: the slots the step kernel adds, and the valid-move count n (the legal
+// kernel's slot; 0 for a move whose list was not built).
+__device__ __forceinline__ int blk_stat_slot(const BlkStepOut &o, int n, int lane) {
+    int v = lane == ST_STEPS ? 1 : lane == ST_NVALID ? n : lane == ST_ERRORS ? o.error
+          : lane == ST_REWARD ? (o.mover + 1) * o.reward : 0;
+    if (o.terminal) {
+        const int q = (lane - ST_WINS) & 3, sq = (lane - ST_SCORE) & 3, rq = (lane - ST_RANK) & 3;
+        v += lane == ST_EPISODES ? 1 : lane == ST_EPLEN ? (int)o.ep_len : lane == ST_NOWIN ? (o.winners == 0)
+           : (lane >= ST_WINS && lane < ST_WINS + 4) ? (o.winners >> q & 1)
+           : (lane >= ST_SCORE && lane < ST_SCORE + 4) ? (int)(o.scores >> (8 * sq) & 0xffu)
+           : (lane >= ST_RANK && lane < ST_RANK + 4) ? (~o.winners >> rq & 1) : 0;
+    }
+    return v;
+}
+
 // ---- K fused random-policy steps with auto-reset: one warp per game, the game stays in shared memory for all K steps.
 // Step t is K x (legal kernel, player -1, auto-reset -> policy_random(step0 + t) -> step kernel, auto-reset) with the
 // list never materialised: blk_enumerate<BLK_SELECT> counts the mover's ids and finds the one at index
@@ -700,30 +732,75 @@ blokus_rollout_kernel(uint4 *__restrict__ st, uint2 *__restrict__ result, crl_u6
     for (int t = 0; t < K; t++) {
         __syncwarp();                                        // the previous step's commit (and the zeroing) is visible
         if (sm.st[85] >> 16 & 1u) blk_new_state(sm, lane);
-        const uint32_t meta = sm.st[85];
-        const int c = (int)(meta >> 8 & 3u);
-        int aid = -1, n = 0;
-        if (!(sm.st[87] >> c & 1u)) {                        // not known to be stuck (w[87]): enumerate
-            const uint32_t r = env_words(seed, first_env + (crl_u64)g, step0 + (uint32_t)t, CRL_TAG_BLOKUS).x;
-            n = blk_enumerate<BLK_SELECT>(sm, c, (int)(meta & 0xffu), sm.st[80 + c], lane, nullptr, 0, r, &aid);
-        }
-        const BlkStepOut o = blk_step_apply(sm, aid, lane, zeroed);
+        int n;
+        const BlkStepOut o = blk_random_move(sm, seed, first_env + (crl_u64)g, step0 + (uint32_t)t, CRL_TAG_BLOKUS, 0, lane,
+                                             zeroed, n);
         rec = blk_result(o);
-        if (stats) {                                         // the slots the legal and step kernels add
-            int v = lane == ST_STEPS ? 1 : lane == ST_NVALID ? n : lane == ST_ERRORS ? o.error
-                  : lane == ST_REWARD ? (o.mover + 1) * o.reward : 0;
-            if (o.terminal) {
-                const int q = (lane - ST_WINS) & 3, sq = (lane - ST_SCORE) & 3, rq = (lane - ST_RANK) & 3;
-                v += lane == ST_EPISODES ? 1 : lane == ST_EPLEN ? (int)o.ep_len : lane == ST_NOWIN ? (o.winners == 0)
-                   : (lane >= ST_WINS && lane < ST_WINS + 4) ? (o.winners >> q & 1)
-                   : (lane >= ST_SCORE && lane < ST_SCORE + 4) ? (int)(o.scores >> (8 * sq) & 0xffu)
-                   : (lane >= ST_RANK && lane < ST_RANK + 4) ? (~o.winners >> rq & 1) : 0;
-            }
-            acc += (crl_u64)(long long)v;
-        }
+        if (stats) acc += (crl_u64)(long long)blk_stat_slot(o, n, lane);     // the slots the legal and step kernels add
     }
     blk_store(sm, st, g, lane);
     if (result && lane == 0) result[g] = rec;
+    if (stats && acc != 0) atomicAdd(stats + (blockIdx.x & (CRL_STAT_ROWS - 1)) * CRL_NSTAT + lane, acc);
+}
+
+// ---- one learner against uniform random opponents (crl_blokus_advance; the rule is stated in
+// include/colosseum_b200_learner.h): one warp per game, like the rollout.  The learner's id, then opponent moves j =
+// 0, 1, ... (blk_random_move on word j & 3 of tag CRL_TAG_OPPONENT + (j >> 2)) until the mover is `seat`; a move that
+// ends the game is recorded and the game restarted at once.  A fresh game cannot end within its first 3 moves (every
+// colour has a move in round 0), so at most 2 x 4 - 2 = 6 opponent moves are made: the loop bound never decides.
+// Record, 8 bytes: int8 learner reward | u8 flags (1 finished, 2 illegal, 4 placed, 8 the learner did not move) |
+// u8 winners | u8 opponent moves, then the finished game's scores (one byte per seat) or 0.  Statistics: lane s
+// accumulates slot s in 64 bits and adds it to the CTA's row once.
+__global__ void __launch_bounds__(32 * BLK_WARPS)
+blokus_advance_kernel(uint4 *__restrict__ st, const int32_t *__restrict__ actions, int seat, uint2 *__restrict__ result,
+                      crl_u64 *stats, long long B, crl_u64 seed, crl_u64 first_env, uint32_t step) {
+    __shared__ BlkSmem smem[BLK_WARPS];
+    const int lane = BLK_WARPS == 1 ? (int)threadIdx.x : (int)(threadIdx.x & 31), wid = BLK_WARPS == 1 ? 0 : (int)(threadIdx.x >> 5);
+    const long long g = (long long)blockIdx.x * BLK_WARPS + wid;
+    if (g >= B) return;
+    BlkSmem &sm = smem[wid];
+    blk_load(sm, st, g, lane);
+    blk_zero_fit(sm, lane);                                  // once: see blokus_rollout_kernel
+    bool zeroed = true;
+    crl_u64 acc = 0;
+    uint32_t flags = 0u, winners = 0u, scores = 0u;
+    int reward = 0, j = 0;
+    // a move that ended the game: record it for the learner (its index in the stable ascending sort of the scores), restart
+    auto finish = [&](const BlkStepOut &o) {
+        flags |= 1u;
+        winners = (uint32_t)o.winners;
+        scores = o.scores;
+        const int ss = (int)(o.scores >> (8 * seat) & 0xffu);
+        reward = 0;
+#pragma unroll
+        for (int q = 0; q < 4; q++) {
+            const int sq = (int)(o.scores >> (8 * q) & 0xffu);
+            reward += (sq < ss || (sq == ss && q < seat)) ? 1 : 0;
+        }
+        blk_new_state(sm, lane);
+    };
+    __syncwarp();
+    if (sm.st[85] >> 16 & 1u) blk_new_state(sm, lane);       // 1. it ended in an earlier call
+    if (actions && (int)(sm.st[85] >> 8 & 3u) == seat) {     // 2. the learner's move
+        const BlkStepOut o = blk_step_apply(sm, actions[g], lane, zeroed);
+        flags |= (uint32_t)(o.error << 1 | o.placed << 2);
+        if (stats) acc += (crl_u64)(long long)blk_stat_slot(o, 0, lane);
+        if (o.terminal) finish(o);
+    } else {
+        flags |= 8u;
+    }
+#pragma unroll 1
+    for (; j < 2 * 4 - 2; j++) {                             // 3. the opponents
+        __syncwarp();                                        // the previous commit is visible
+        if ((int)(sm.st[85] >> 8 & 3u) == seat) break;
+        int n;
+        const BlkStepOut o = blk_random_move(sm, seed, first_env + (crl_u64)g, step, CRL_TAG_OPPONENT + (uint32_t)(j >> 2), j & 3,
+                                             lane, zeroed, n);
+        if (stats) acc += (crl_u64)(long long)blk_stat_slot(o, n, lane);
+        if (o.terminal) finish(o);
+    }
+    blk_store(sm, st, g, lane);
+    if (lane == 0) result[g] = make_uint2(((uint32_t)reward & 0xffu) | flags << 8 | winners << 16 | (uint32_t)j << 24, scores);
     if (stats && acc != 0) atomicAdd(stats + (blockIdx.x & (CRL_STAT_ROWS - 1)) * CRL_NSTAT + lane, acc);
 }
 

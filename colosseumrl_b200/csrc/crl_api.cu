@@ -806,4 +806,42 @@ int crl_tron_rollout_avoid(void *state, uint8_t *result, int64_t *stats, uint64_
     return tron_rollout_launch(s, state, result, stats, seed, first_env, step0, K, B, avoid_mask, noise_q16, stream);
 }
 
+/* ------------------------------------------------------------------------------------------- one learner */
+
+int crl_ttt_advance(void *state, const int8_t *actions, int seat, uint8_t *result, uint32_t *valid_after, int64_t *stats,
+                    uint64_t seed, uint64_t first_env, uint32_t step, int64_t B, int n, crl_stream_t stream) {
+    TTTParams prm;
+    int rc = ttt_params(n, prm);
+    if (rc) return rc;
+    if (!state || !result) return fail(CRL_ERR_ARG, "crl_ttt_advance: null state or result");
+    if (B < 0) return fail(CRL_ERR_ARG, "crl_ttt_advance: negative batch");
+    if (seat < 0 || seat >= n) return fail(CRL_ERR_ARG, "crl_ttt_advance: seat must satisfy 0 <= seat < n");
+    if (B == 0) return CRL_OK;
+    if (B >= (int64_t)1 << 31) return fail(CRL_ERR_UNSUPPORTED, "crl_ttt_advance: batch too large for one launch");
+    if ((uintptr_t)state & 15) return fail(CRL_ERR_ARG, "crl_ttt_advance: state must be 16-byte aligned");
+    if (((uintptr_t)result | (uintptr_t)valid_after) & 3)
+        return fail(CRL_ERR_ARG, "crl_ttt_advance: result and valid_after must be 4-byte aligned");
+    return dispatch<2, 3, 4>(n, [&](auto NP) {
+        return dispatch<true, false>(stats != nullptr, [&](auto STATS) {
+            return launch("ttt_advance_kernel", ttt_advance_kernel<NP, STATS>, {ttt_blocks(B), 256}, stream,
+                          (uint4 *)state, actions, seat, (uint32_t *)result, valid_after, (crl_u64 *)stats, (int)B,
+                          (crl_u64)seed, (crl_u64)first_env, step);
+        });
+    });
+}
+
+int crl_blokus_advance(void *state, const int32_t *actions, int seat, uint8_t *result, int64_t *stats, uint64_t seed,
+                       uint64_t first_env, uint32_t step, int64_t B, crl_stream_t stream) {
+    if (!state || !result) return fail(CRL_ERR_ARG, "crl_blokus_advance: null state or result");
+    if (B < 0) return fail(CRL_ERR_ARG, "crl_blokus_advance: negative batch");
+    if (seat < 0 || seat > 3) return fail(CRL_ERR_ARG, "crl_blokus_advance: seat must satisfy 0 <= seat < 4");
+    if (B == 0) return CRL_OK;
+    if ((uintptr_t)state & 15) return fail(CRL_ERR_ARG, "crl_blokus_advance: state must be 16-byte aligned");
+    if ((uintptr_t)result & 7) return fail(CRL_ERR_ARG, "crl_blokus_advance: result must be 8-byte aligned");
+    if ((uintptr_t)actions & 3) return fail(CRL_ERR_ARG, "crl_blokus_advance: actions must be 4-byte aligned");
+    return launch("blokus_advance_kernel", blokus_advance_kernel, {blocks_for(B, BLK_WARPS), 32 * BLK_WARPS}, stream,
+                  (uint4 *)state, actions, seat, (uint2 *)result, (crl_u64 *)stats, B, (crl_u64)seed, (crl_u64)first_env,
+                  step);
+}
+
 }  // extern "C"

@@ -7,6 +7,7 @@
 #define CRL_TAG_BLOKUS 2u
 #define CRL_TAG_TTT 3u
 #define CRL_TAG_TRON_AVOID 4u       // Tron avoid policy: seats 0..3 use tag 4, seats 4..7 tag 5
+#define CRL_TAG_OPPONENT 6u         // TTT / Blokus random opponents of crl_*_advance: moves 0..3 use tag 6, 4..7 tag 7
 
 __device__ __forceinline__ uint4 philox4x32_10(uint32_t c0, uint32_t c1, uint32_t c2, uint32_t c3,
                                                uint32_t k0, uint32_t k1) {

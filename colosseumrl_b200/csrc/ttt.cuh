@@ -531,3 +531,77 @@ __global__ void ttt_pack_kernel(uint4 *__restrict__ st, long long B, TTTParams p
     }
     st[e] = ttt_encode(s);
 }
+
+// ---- one learner against uniform random opponents (crl_ttt_advance; the rule is stated in
+// include/colosseum_b200_learner.h).  One thread per environment, grid-stride with a block-uniform trip count like the
+// rollout kernel, because the statistics flushes are warp-collective.  Every lane runs the same 2NP - 2 opponent
+// slots; slot j is active while the game's mover is not `seat` (a game is restarted as soon as a move ends it, so the
+// active slots are exactly the first j and their index is the opponent move index of the rule).  The pick is a plain
+// `%`: ttt_mod_small shuffles, and the active slots of the lanes differ.
+//   Statistics bound (the packed fields of TTTStatAcc, 32 lanes per flush): an environment is at most 2NP - 1
+//   env-steps (the learner's move and 2NP - 2 opponent moves), each with nvalid <= CELLS, with at most one finished
+//   episode.  Flushed once per environment, the 12-bit nvalid field would hold up to 32 x 27 x 7 = 6048 for NP = 4,
+//   so 4-player flushes twice: after the learner's move and slots 0..2 (<= 4 env-steps: nvalid <= 3456, steps <= 128,
+//   reward + bias <= 8 x 128) and after slots 3..5 (<= 3).  NP = 3 (<= 5 env-steps: nvalid <= 2400) and NP = 2
+//   (<= 3: 864) flush once.  Episodes, wins and episode lengths (<= 31 x 32) are bounded by one episode per lane.
+template <int NP, bool STATS>
+__global__ void __launch_bounds__(256)
+ttt_advance_kernel(uint4 *__restrict__ state, const int8_t *__restrict__ actions, int seat, uint32_t *__restrict__ result,
+                   uint32_t *__restrict__ valid_after, crl_u64 *stats, int B, crl_u64 seed, crl_u64 first_env,
+                   uint32_t step) {
+    constexpr int SLOTS = 2 * NP - 2;
+    crl_u64 *const row = STATS ? stats + (blockIdx.x & (CRL_STAT_ROWS - 1)) * CRL_NSTAT : nullptr;
+    const uint32_t lane_const = TTT_STAT_LANE[threadIdx.x & 31];
+    TTTStatAcc acc;
+    acc.clear();
+    // unsigned: B < 2^31 and stride < 2^31, so e0 + stride stays below 2^32 at the last trip
+    const uint32_t stride = gridDim.x * blockDim.x, first = blockIdx.x * blockDim.x;
+    for (uint32_t e0 = first; e0 < (uint32_t)B; e0 += stride) {
+        const uint32_t e = e0 + threadIdx.x;
+        const bool valid = e < (uint32_t)B;
+        TTTEnv s;
+        ttt_new_state(s);
+        if (valid) ttt_decode(s, ld_stream(state + e));
+        if (ttt_is_terminal<NP>(s)) ttt_new_state(s);                    // 1. it ended in an earlier call
+        uint32_t flags = 0u, winners = 0u;
+        int reward = 0, j = 0;
+        TTTOut o;
+        ttt_zero_out(o);
+        // a move that ended the game: record it for the learner, restart
+        auto finish = [&]() {
+            flags |= 1u;
+            winners = (uint32_t)o.winners;
+            reward = s.winner1 == 0 ? 0 : (s.winner1 - 1 == seat ? 1 : -1);
+            ttt_new_state(s);
+        };
+        if (actions && s.mover == seat) {                                // 2. the learner's move
+            ttt_step_env<NP>(s, valid ? (int)actions[e] : -1, o);
+            flags |= (uint32_t)(o.error << 1 | o.placed << 2);
+            if (STATS && valid) acc.add<NP>(o, seat, s.ep_len);
+            if (o.terminal) finish();
+        } else {
+            flags |= 8u;
+        }
+        uint4 w = make_uint4(0u, 0u, 0u, 0u);
+#pragma unroll
+        for (int k = 0; k < SLOTS; k++) {                                // 3. the opponents
+            if (STATS && NP == 4 && k == NP - 1) acc.flush<NP, true>(nullptr, lane_const, row);
+            if (s.mover != seat) {
+                if ((k & 3) == 0) w = env_words(seed, first_env + (crl_u64)e, step, CRL_TAG_OPPONENT + (uint32_t)(k >> 2));
+                const uint32_t r = (k & 3) == 0 ? w.x : (k & 3) == 1 ? w.y : (k & 3) == 2 ? w.z : w.w;
+                const uint32_t empty = ~(s.c[0] | s.c[1] | s.c[2] | s.c[3]) & TTTGeo<NP>::CELLMASK;   // non-terminal: >= 1
+                const int mover = s.mover;
+                ttt_step_env<NP>(s, 31 - __clz((int)ttt_kth_bit_onehot(empty, r % (uint32_t)__popc(empty))), o);
+                if (STATS && valid) acc.add<NP>(o, mover, s.ep_len);
+                if (o.terminal) finish();
+                j++;
+            }
+        }
+        if (STATS) acc.flush<NP, true>(nullptr, lane_const, row);
+        if (valid) {
+            st_stream(state + e, ttt_encode(s));
+            result[e] = ((uint32_t)reward & 0xffu) | flags << 8 | winners << 16 | (uint32_t)j << 24;
+            if (valid_after) valid_after[e] = ~(s.c[0] | s.c[1] | s.c[2] | s.c[3]) & TTTGeo<NP>::CELLMASK;
+        }
+    }
+}

@@ -171,6 +171,22 @@ class _BatchedTicTacToe(BatchedBaseEnvironment):
                                               self.N_PLAYERS, self._stream))
         return state
 
+    def advance(self, state: TTTBatchState, actions, seat: int, step: int) -> torch.Tensor:
+        """One learner move against uniform random opponents, in place (crl_ttt_advance; the rule is stated in
+        include/colosseum_b200_learner.h): the learner at `seat` plays `actions` (int8 [B] cells; None: it does not
+        move), then the other seats play until `seat` is to move again, restarting finished games.  Returns the record
+        uint8 [B, 4]: int8 learner reward | flags (1 a game finished, 2 illegal, 4 placed, 8 the learner did not move) |
+        winners mask of the finished game | opponent moves.  state.valid becomes the learner's valid actions."""
+        a = None if actions is None else self._dev(actions, torch.int8)
+        if state.valid is None:
+            state.valid = torch.empty((self.batch,), dtype=torch.int32, device=self.device)
+        rec = self._new_result((self.batch, 4))
+        self._check(self._lib.crl_ttt_advance(state.packed.data_ptr(), None if a is None else a.data_ptr(), int(seat),
+                                              rec.data_ptr(), state.valid.data_ptr(), self._stats_ptr, self.seed,
+                                              self.first_env_id, int(step), self.batch, self.N_PLAYERS, self._stream))
+        state.result = None                    # the record of an earlier step no longer describes `state`
+        return rec
+
 
 class BatchedTicTacToe2PlayerEnv(_BatchedTicTacToe):
     N_PLAYERS = 2

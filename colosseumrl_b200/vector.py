@@ -117,3 +117,68 @@ class SingleAgentVectorEnv:
         info = {"players": players.clone(), "winners": winners.clone(), "terminal": terminal.clone()}
         self.env.reset_where(self.state, done)
         return self._observe(), reward, done, info
+
+
+class SingleAgentTurnVectorEnv:
+    """One learner seat against uniform random opponents on the device, for the turn-based games (Tic Tac Toe, Blokus).
+    Each step is ONE advance launch (the learner's move, then every opponent move up to the learner's next turn, with
+    finished games restarted) plus the observation:
+
+        venv = SingleAgentTurnVectorEnv(BatchedBlokusEnvironment(batch=1024), seat=1, perspective=True)
+        obs = venv.reset()                           # the seat's view (Blokus: rotated for the seat)
+        counts, ids = venv.valid_actions()           # Blokus: the seat's lists (perspective: in the rotated frame)
+        obs, reward, done, info = venv.step(actions)  # reward int8 [B]; done uint8 [B]
+
+    The rule is this engine's definition (include/colosseum_b200_learner.h).  Every returned game is the learner's
+    turn; `done` marks the step in which a game finished, and that game has already been restarted (and played up to
+    the learner's turn), so the observation describes the game the next action applies to.  reward: Tic Tac Toe +1 /
+    -1 / 0 for a win / loss / draw of the learner, Blokus its index in the stable ascending sort of the final scores;
+    0 while a game goes on.  info: "winners" (mask of the finished game), "opponent_moves", "illegal" and, for Blokus,
+    "scores" (uint8 [B, 4], the finished game's).  The opponents' Philox step is a counter kept here (reset() sets it to
+    0, and reset() itself is step 0)."""
+
+    def __init__(self, env, seat: int = 0, perspective: bool = False):
+        if not hasattr(env, "advance"):
+            raise TypeError("SingleAgentTurnVectorEnv needs a Tic Tac Toe or Blokus environment")
+        if not 0 <= seat < env.max_players:
+            raise ValueError("seat must be in [0, %d)" % env.max_players)
+        self.blokus = hasattr(env, "player_perspective_valid_actions")
+        if perspective and not self.blokus:
+            raise ValueError("perspective=True exists for Blokus only")
+        self.env, self.seat, self.perspective = env, int(seat), bool(perspective)
+        self.state, self.t = None, 0
+
+    @property
+    def num_envs(self) -> int:
+        return self.env.batch
+
+    def _observe(self) -> Dict[str, torch.Tensor]:
+        return self.env.state_to_observation(self.state, self.seat)
+
+    def reset(self) -> Dict[str, torch.Tensor]:
+        self.state, _ = self.env.new_state()
+        self.env.advance(self.state, None, self.seat, 0)
+        self.t = 1
+        return self._observe()
+
+    def valid_actions(self):
+        """Tic Tac Toe: the empty-cell mask int32 [B]; Blokus: (counts, ids) of the seat (perspective=True: rotated).
+        Fresh tensors: the next step() does not change them."""
+        if not self.blokus:
+            return self.env.valid_actions(self.state).clone()     # (the cached mask is rewritten by the next advance)
+        if self.perspective:
+            return self.env.player_perspective_valid_actions(self.state, self.seat)
+        return self.env.valid_actions(self.state, self.seat, count_stats=False)
+
+    def step(self, actions):
+        """actions: the learner's, int8 [B] cells (Tic Tac Toe) or int32 [B] ids (Blokus; perspective=True: in the
+        seat's rotated frame).  Returns (observation, reward int8 [B], done uint8 [B], info)."""
+        if self.perspective:
+            from .blokus import player_perspective_action_to_real
+            actions = player_perspective_action_to_real(self.env._dev(actions, torch.int32), self.seat)
+        rec = self.env.advance(self.state, actions, self.seat, self.t)
+        self.t += 1
+        info = {"winners": rec[:, 2], "opponent_moves": rec[:, 3], "illegal": (rec[:, 1] >> 1) & 1}
+        if self.blokus:
+            info["scores"] = rec[:, 4:8]
+        return self._observe(), rec[:, 0].view(torch.int8), rec[:, 1] & 1, info

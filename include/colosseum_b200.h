@@ -258,4 +258,6 @@ int crl_blokus_pack(void *state, const int8_t *board, const uint8_t *pieces, con
 
 /* device-side Tron opponents (the avoid policy and its fused rollout) */
 #include "colosseum_b200_tron_policy.h"
+/* one learner seat against device-side random opponents (Tic Tac Toe, Blokus) */
+#include "colosseum_b200_learner.h"
 #endif
