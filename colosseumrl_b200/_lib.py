@@ -82,6 +82,13 @@ LEARNER_SIGNATURES = {
     "crl_blokus_advance": (_int, [_vp, _vp, _int, _vp, _vp, _u64, _u64, _u32, _i64, _vp]),
 }
 
+# ... and of the companion header include/colosseum_b200_placement.h (Blokus placements: masks, placement -> action id)
+PLACEMENT_SIGNATURES = {
+    "crl_blokus_placement_mask": (_int, [_vp, _int, _int, _vp, _vp, _i64, _int, _vp]),
+    "crl_blokus_placement_to_action": (_int, [_vp, _int, _int, _vp, _vp, _i64, _int, _vp]),
+    "crl_blokus_shape_table": (_int, [_vp, _vp, _vp, _vp]),
+}
+
 
 class CrlError(RuntimeError):
     pass
@@ -89,7 +96,8 @@ class CrlError(RuntimeError):
 
 def declare(lib):
     """Attach restype/argtypes for every exported symbol; raises if one is missing."""
-    for name, (res, args) in list(SIGNATURES.items()) + list(TRON_POLICY_SIGNATURES.items()) + list(LEARNER_SIGNATURES.items()):
+    tables = (SIGNATURES, TRON_POLICY_SIGNATURES, LEARNER_SIGNATURES, PLACEMENT_SIGNATURES)
+    for name, (res, args) in [item for table in tables for item in table.items()]:
         fn = getattr(lib, name)  # AttributeError if the symbol is not exported
         fn.restype = res
         fn.argtypes = args

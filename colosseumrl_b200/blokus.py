@@ -60,6 +60,69 @@ def player_perspective_action_to_real(ids, player: int):
     return _rotate_action_ids(ids, int(player), True)
 
 
+# ---- placements (include/colosseum_b200_placement.h) -----------------------------------------------------------------
+# A placement is p = s * 400 + y * 20 + x: oriented shape s (0..90, the engine's shape order: by size, then piece, then
+# first appearance in ORIENTATIONS order) with the top-left corner of its bounding box at (x, y); -1 is a pass.  It is
+# legal for a player iff the player holds the piece of s, every cell is on the board and allowed, and a cell is one of
+# the player's anchors (round 0: the corner) -- exactly the placements of the ids in valid_actions' list.  In a
+# player's perspective frame (the frame of state_to_observation(state, player)) a placement is the rotated cell set.
+NUM_SHAPES = 91
+NUM_PLACEMENTS = NUM_SHAPES * 400
+ILLEGAL_ACTION = 21 * 16000             # what an illegal placement converts to: flagged and applied as a pass by a step
+
+
+def shape_tables() -> Dict[str, "np.ndarray"]:
+    """The library's shape tables (crl_blokus_shape_table), read once: "piece" [91], "cells" [91, 5, 2] ((dx, dy), -1
+    past the shape's size), "rotation" [91, 4] (the image in player q's frame) and "action_shape" [21, 40, 3]
+    ((shape, dx, dy) per piece and orientation * 5 + shift; -1 for shifts past the piece's size)."""
+    global _SHAPE_TABLES
+    if _SHAPE_TABLES is None:
+        import numpy as np
+        t = {"piece": np.zeros(91, np.int32), "cells": np.zeros((91, 5, 2), np.int32),
+             "rotation": np.zeros((91, 4), np.int32), "action_shape": np.zeros((21, 40, 3), np.int32)}
+        n = _lib.load().crl_blokus_shape_table(*(t[k].ctypes.data for k in ("piece", "cells", "rotation", "action_shape")))
+        assert n == NUM_SHAPES
+        # id -> placement of the id's own frame, over all 336 000 ids
+        a = t["action_shape"]
+        ids = np.arange(ILLEGAL_ACTION)
+        ok, cell, piece = ids % 40, (ids // 40) % 400, ids // 16000
+        s, dx, dy = a[piece, ok, 0], a[piece, ok, 1], a[piece, ok, 2]
+        x, y = cell % 20 - dx, cell // 20 - dy
+        t["id_placement"] = np.where((s >= 0) & (x >= 0) & (y >= 0), s * 400 + y * 20 + x, -1).astype(np.int32)
+        _SHAPE_TABLES = t
+    return _SHAPE_TABLES
+
+
+_SHAPE_TABLES = None
+
+
+def action_to_placement(ids, player: Optional[int] = None):
+    """Action id -> placement, on ints, numpy arrays or integer tensors; -1 (pass) stays -1.  With `player`, the
+    placement in that player's perspective frame: action_to_placement(id, r) == action_to_placement(
+    real_action_to_player_perspective(id, r)).  Ids that no list can hold (a shift past the piece's size, a corner off
+    the board) give -1 as well."""
+    if player is not None:
+        ids = real_action_to_player_perspective(ids, player)
+    lut = shape_tables()["id_placement"]
+    if isinstance(ids, int):
+        return int(lut[ids]) if 0 <= ids < ILLEGAL_ACTION else -1
+    if isinstance(ids, torch.Tensor):
+        t = torch.as_tensor(lut, device=ids.device)
+        inside = (ids >= 0) & (ids < ILLEGAL_ACTION)
+        return torch.where(inside, t[ids.clamp(0, ILLEGAL_ACTION - 1).long()], torch.full_like(t[:1], -1)).to(ids.dtype)
+    import numpy as np
+    ids = np.asarray(ids)
+    inside = (ids >= 0) & (ids < ILLEGAL_ACTION)
+    return np.where(inside, lut[np.clip(ids, 0, ILLEGAL_ACTION - 1)], -1).astype(ids.dtype)
+
+
+def placement_mask(words: torch.Tensor) -> torch.Tensor:
+    """valid_placements' words int32 [B, 91, 20] -> bool [B, 36 400], entry p = s * 400 + y * 20 + x set iff placement
+    p is legal: ready for logits.masked_fill(~mask, float("-inf"))."""
+    bits = torch.arange(20, dtype=torch.int32, device=words.device)
+    return ((words.unsqueeze(-1) >> bits) & 1).bool().reshape(words.shape[0], NUM_PLACEMENTS)
+
+
 @dataclass
 class BlokusBatchState:
     packed: torch.Tensor                        # int32 [B, 22, 4]: 352 bytes per game
@@ -125,6 +188,33 @@ class BatchedBlokusEnvironment(BatchedBaseEnvironment):
                                                ids.shape[1], self._stats_ptr if count_stats else None, self.batch,
                                                self.flags, self._stream))
         return counts, ids
+
+    def valid_placements(self, state: BlokusBatchState, player: int = -1, perspective: bool = False,
+                         out: Optional[Tuple[torch.Tensor, torch.Tensor]] = None):
+        """Legal placements of `player` (-1: each game's mover) as (counts int32 [B], words int32 [B, 91, 20]): bit x of
+        words[g, s, y] is set iff placement s * 400 + y * 20 + x is legal (placement_mask unpacks it).  perspective:
+        placements in the player's rotated frame (that of state_to_observation(state, player)).  One
+        crl_blokus_placement_mask launch; no action list is built."""
+        if out is None:
+            out = (torch.empty((self.batch,), dtype=torch.int32, device=self.device),
+                   torch.empty((self.batch, NUM_SHAPES, 20), dtype=torch.int32, device=self.device))
+        counts, words = out
+        self._check(self._lib.crl_blokus_placement_mask(state.packed.data_ptr(), int(player), int(bool(perspective)),
+                                                        words.data_ptr(), counts.data_ptr(), self.batch, self.flags,
+                                                        self._stream))
+        return counts, words
+
+    def placements_to_actions(self, state: BlokusBatchState, placements, player: int = -1,
+                              perspective: bool = False) -> torch.Tensor:
+        """Placements (int32 [B], -1 = pass; perspective: in the player's rotated frame) -> action ids int32 [B] in the
+        board frame: the first id of the player's valid list with that placement, -1 for -1, ILLEGAL_ACTION for an
+        illegal or out-of-range placement (a step flags it and applies a pass)."""
+        placements = self._dev(placements, torch.int32)
+        actions = torch.empty((self.batch,), dtype=torch.int32, device=self.device)
+        self._check(self._lib.crl_blokus_placement_to_action(state.packed.data_ptr(), int(player), int(bool(perspective)),
+                                                             placements.data_ptr(), actions.data_ptr(), self.batch,
+                                                             self.flags, self._stream))
+        return actions
 
     def is_valid_action(self, state: BlokusBatchState, player: int, action) -> torch.Tensor:
         """is_valid_action (:667-719): uint8 [B], 1 iff action[g] is in `player`'s valid list (-1 / '' is not).

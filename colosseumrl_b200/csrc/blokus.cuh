@@ -950,3 +950,181 @@ __global__ void blokus_pack_kernel(uint4 *__restrict__ st4, long long B, const i
     }
     st[idx] = v;
 }
+
+// ---- placements (include/colosseum_b200_placement.h): placement p = s * 400 + y * 20 + x, shape s with the top-left
+// corner of its bounding box at (x, y).  (s, x, y) is legal for player c  <=>  c holds the piece of s, FIT_s[(x, y)]
+// (every cell allowed) and a cell is an anchor:  mask_s = FIT_s & OR_k shift(ANC, -cell_k)  -- blk_any_pass with a
+// store per row instead of an OR-reduction, and no emission phase at all.
+#define BLK_NPLACEMENT (BLK_NSHAPE * 400)
+#define BLK_ILLEGAL_ACTION (BLK_NPIECE * 16000)     // in no valid list: the step kernels flag it and apply a pass
+#define BLK_MASK_VEC (BLK_NSHAPE * 20 / 4)          // uint4 per game of the mask uint32[91][20] (7 280 bytes)
+
+// shape -> its image in player q's rotated frame (q = 0..3), for blokus_placement_to_action_kernel.  Passed BY VALUE
+// (kernel parameter space), so it adds nothing to the constant banks the other kernels address.
+struct BlkRotTab {
+    uint8_t img[4][BLK_NSHAPE + 1];
+};
+
+// Row `lane` (< 20; 0 in lanes 20..31) of a 20 x 20 bit board -> row `lane` of the board in player r's frame (r = 1..3),
+// the frame of blokus_observe_kernel: board cell (x, y) lands on (19 - y, x), (19 - x, 19 - y), (y, 19 - x).  With the
+// transpose T (T[j] bit i = B[i] bit j: 20 ballots) the rotated rows are rev(T[y]), rev(B[19 - y]) and T[19 - y].
+__device__ __forceinline__ uint32_t blk_rotate_row(uint32_t v, int r, int lane) {
+    if (r & 1) {
+        uint32_t t = 0u;
+#pragma unroll
+        for (int j = 0; j < 20; j++) {
+            const uint32_t b = __ballot_sync(0xffffffffu, (v >> j) & 1u);
+            t = lane == j ? b : t;
+        }
+        v = t;
+    }
+    v = __shfl_sync(0xffffffffu, v, r == 1 ? lane : (19 - lane) & 31);
+    if (r != 3) v = __brev(v) >> 12;
+    return lane < 20 ? v : 0u;
+}
+
+// Mask rows of the shapes [s0, s1), lanes = shapes: row y of shape s is FIT_s[y] & OR_k (anc[y + dy_k] >> dx_k) for a
+// shape whose piece is held and whose board `flags` marks as built and non-empty (bit lane), zero rows otherwise.  The
+// lane writes its shape's 80 contiguous bytes with five 128-bit stores and returns their popcount.  anc: the anchor
+// rows with rows 20..23 zero (shapes are at most 5 rows tall); off: bit of column 0 in these FIT boards.
+__device__ __forceinline__ int blk_mask_pass(const BlkSmem &sm, const uint32_t *anc, int s0, int s1, uint32_t flags,
+                                             uint32_t inv, uint32_t off, uint4 *__restrict__ out, int lane) {
+    if (s0 + lane >= s1) return 0;
+    const uint4 t = BLK_SHAPE_TAB_G[s0 + lane];
+    uint4 *o = out + (s0 + lane) * 5;
+    if (!((inv >> (t.w >> 16 & 31u) & 1u) && (flags >> lane & 1u))) {
+#pragma unroll
+        for (int q = 0; q < 5; q++) o[q] = make_uint4(0u, 0u, 0u, 0u);
+        return 0;
+    }
+    const uint32_t *f = (const uint32_t *)((const char *)sm.F + (t.w & 0xffffu));        // own row 4 (y = 0)
+    const uint32_t *a0 = anc + (t.z >> 3 & 7u), *a1 = anc + (t.z >> 9 & 7u), *a2 = anc + (t.z >> 15 & 7u);
+    const uint32_t *a3 = anc + (t.z >> 21 & 7u), *a4 = anc + (t.z >> 27 & 7u);           // (short shapes repeat cell 0)
+    const uint32_t d0 = t.z & 7u, d1 = t.z >> 6 & 7u, d2 = t.z >> 12 & 7u, d3 = t.z >> 18 & 7u, d4 = t.z >> 24 & 7u;
+    int cnt = 0;
+#pragma unroll
+    for (int q = 0; q < 5; q++) {
+        uint32_t m[4];
+#pragma unroll
+        for (int i = 0; i < 4; i++) {
+            const int r = 4 * q + i;
+            const uint32_t d = (a0[r] >> d0) | (a1[r] >> d1) | (a2[r] >> d2) | (a3[r] >> d3) | (a4[r] >> d4);
+            m[i] = (f[r] >> off) & d & BLK_ROWMASK;
+            cnt += __popc(m[i]);
+        }
+        o[q] = make_uint4(m[0], m[1], m[2], m[3]);
+    }
+    return cnt;
+}
+
+// ---- legal-placement masks: one warp per game, as the legal kernel.  A and ANC of the player (rotated into its frame
+// for frame 1: legality only asks which cells are allowed and which are anchors, so it is invariant under the rotation),
+// the tree passes of the legal kernel, and one mask pass per range of shapes (the <= 4-cell shapes, then each pentomino
+// group).  player < 0: the game's mover.
+__global__ void __launch_bounds__(32 * BLK_WARPS)
+blokus_placement_mask_kernel(const uint4 *__restrict__ st, uint4 *__restrict__ mask, int32_t *__restrict__ counts,
+                             long long B, int player, int frame, int flags) {
+    __shared__ BlkSmem smem[BLK_WARPS];
+    __shared__ uint32_t sanc[BLK_WARPS][24];                 // anchor rows, rows 20..23 zero
+    const int lane = BLK_WARPS == 1 ? (int)threadIdx.x : (int)(threadIdx.x & 31), wid = BLK_WARPS == 1 ? 0 : (int)(threadIdx.x >> 5);
+    const long long g = (long long)blockIdx.x * BLK_WARPS + wid;
+    if (g >= B) return;
+    BlkSmem &sm = smem[wid];
+    uint32_t *anc = sanc[wid];
+    blk_load(sm, st, g, lane);
+    if ((flags & CRL_FLAG_AUTO_RESET) && (sm.st[85] >> 16 & 1u)) blk_new_state(sm, lane);
+    const uint32_t meta = sm.st[85];
+    const int c = player >= 0 ? player : (int)(meta >> 8 & 3u);
+    const uint32_t inv = sm.st[80 + c];
+    uint4 *out = mask + g * BLK_MASK_VEC;
+    uint32_t rows = 0u;
+    if (!(sm.st[87] >> c & 1u) && inv != 0u) rows = (uint32_t)blk_allowed_and_anchors<false>(sm, c, (int)(meta & 0xffu), lane);
+    int cnt = 0;
+    if (rows == 0u) {                                        // no anchor, no piece or known to be stuck: no placement
+        for (int i = lane; i < BLK_MASK_VEC; i += 32) out[i] = make_uint4(0u, 0u, 0u, 0u);
+    } else {
+        uint32_t a = lane < 20 ? sm.A[lane] >> 4 : 0u, an = lane < 20 ? sm.anc[lane] : 0u;
+        const int r = frame ? c : 0;
+        if (r) {
+            a = blk_rotate_row(a, r, lane);
+            an = blk_rotate_row(an, r, lane);
+            if (lane < 24) sm.A[lane] = a << 4;
+        }
+        if (lane < 24) anc[lane] = an;
+        blk_zero_fit(sm, lane);
+        __syncwarp();
+        uint32_t ne = blk_tree_root(sm, lane);
+        ne |= blk_tree_pass_le4(sm, ne, inv, lane);
+        cnt = blk_mask_pass(sm, anc, 0, BLK_NSHAPE_LE4, ne, inv, BLK_OFF_LE4, out, lane);
+#pragma unroll 1
+        for (int gi = 0; gi < BLK_NGROUP; gi++) {
+            const bool held = (inv & ((1u << BLK_GROUP_P0[gi + 1]) - (1u << BLK_GROUP_P0[gi]))) != 0u;
+            const uint32_t ne5 = held ? blk_tree_group(sm, gi, ne, inv, lane) : 0u;
+            cnt += blk_mask_pass(sm, anc, BLK_GROUP_S0[gi], BLK_GROUP_S0[gi + 1], ne5, inv, BLK_OFF_PENT, out, lane);
+        }
+    }
+    cnt = __reduce_add_sync(0xffffffffu, cnt);
+    if (counts && lane == 0) counts[g] = cnt;
+}
+
+// ---- placement -> canonical action id: one warp per game, every lane computes the same (warp-uniform) answer.  A
+// frame-1 placement is mapped back to the board frame (the inverse of player r's rotation is player 4 - r's); held,
+// fit and anchor are checked on the A and ANC rows as blk_validate checks an id.  The id is the first one of the
+// reference's list with this placement: the anchor is the row-major first anchored cell, the orientation the lowest
+// one of the piece whose shape is s, the shift the index of the anchor's cell in that orientation.
+__global__ void __launch_bounds__(32 * BLK_WARPS)
+blokus_placement_to_action_kernel(const uint4 *__restrict__ st, const int32_t *__restrict__ placements,
+                                  int32_t *__restrict__ actions, long long B, int player, int frame, int flags,
+                                  BlkRotTab rot) {
+    __shared__ BlkSmem smem[BLK_WARPS];
+    const int lane = BLK_WARPS == 1 ? (int)threadIdx.x : (int)(threadIdx.x & 31), wid = BLK_WARPS == 1 ? 0 : (int)(threadIdx.x >> 5);
+    const long long g = (long long)blockIdx.x * BLK_WARPS + wid;
+    if (g >= B) return;
+    BlkSmem &sm = smem[wid];
+    blk_load(sm, st, g, lane);
+    if ((flags & CRL_FLAG_AUTO_RESET) && (sm.st[85] >> 16 & 1u)) blk_new_state(sm, lane);
+    const uint32_t meta = sm.st[85];
+    const int c = player >= 0 ? player : (int)(meta >> 8 & 3u);
+    const int p = placements[g];
+    int aid = p == -1 ? -1 : BLK_ILLEGAL_ACTION;
+    if (p >= 0 && p < BLK_NPLACEMENT && !(sm.st[87] >> c & 1u)) {
+        int s = p / 400, y = (p - 400 * s) / 20, x = p % 20;
+        uint32_t cells = BLK_SHAPE_CELLS[s];
+        int w1 = 0, h1 = 0;                                  // bounding box - 1
+#pragma unroll
+        for (int i = 0; i < 5; i++) {
+            w1 = max(w1, (int)(cells >> (6 * i) & 7u));
+            h1 = max(h1, (int)(cells >> (6 * i + 3) & 7u));
+        }
+        const bool on = x + w1 <= 19 && y + h1 <= 19;
+        const int q = (4 - (frame ? c : 0)) & 3;
+        if (on && q) {
+            const int x0 = q == 1 ? 19 - h1 - y : q == 2 ? 19 - w1 - x : y;
+            const int y0 = q == 1 ? x : q == 2 ? 19 - h1 - y : 19 - w1 - x;
+            s = rot.img[q][s];
+            x = x0;
+            y = y0;
+            cells = BLK_SHAPE_CELLS[s];
+        }
+        const int pc = (int)(BLK_SHAPE_TAB_G[s].w >> 16 & 31u);
+        if (on && (sm.st[80 + c] >> pc & 1u)) {
+            blk_allowed_and_anchors<false>(sm, c, (int)(meta & 0xffu), lane);
+            bool fit = true;
+            int first = 400;                                 // row-major index of the first anchored cell
+#pragma unroll
+            for (int i = 0; i < 5; i++) {
+                const int cx = x + (int)(cells >> (6 * i) & 7u), cy = y + (int)(cells >> (6 * i + 3) & 7u);
+                fit = fit && (sm.A[cy] >> (cx + 4) & 1u);
+                if (sm.anc[cy] >> cx & 1u) first = min(first, 20 * cy + cx);
+            }
+            if (fit && first < 400) {
+                const int ay = first / 20, ax = first - 20 * ay, size = BLK_PIECE_SIZE[pc], id0 = BLK_PIECE_ID0[pc];
+                const uint32_t key = (uint32_t)s | (uint32_t)(ax - x) << 7 | (uint32_t)(ay - y) << 10;
+                int j = 0;                                   // ids of the piece in the order o * size + k
+                while (j < 8 * size && (BLK_ID_TAB[id0 + j] & 0x1fffu) != key) j++;
+                if (j < 8 * size) aid = pc * 16000 + first * 40 + (int)(BLK_ID_TAB[id0 + j] >> 13);   // (always found)
+            }
+        }
+    }
+    if (lane == 0) actions[g] = aid;
+}

@@ -845,3 +845,54 @@ int crl_blokus_advance(void *state, const int32_t *actions, int seat, uint8_t *r
 }
 
 }  // extern "C"
+
+/* ------------------------------------------------------------------------------------------- Blokus placements */
+
+extern "C" {
+
+int crl_blokus_placement_mask(const void *state, int player, int frame, uint32_t *mask, int32_t *counts, int64_t B,
+                              int flags, crl_stream_t stream) {
+    if (!state || !mask || B < 0 || player > 3) return fail(CRL_ERR_ARG, "crl_blokus_placement_mask: bad argument");
+    if (frame != 0 && frame != 1) return fail(CRL_ERR_ARG, "crl_blokus_placement_mask: frame must be 0 or 1");
+    if (B == 0) return CRL_OK;
+    if (((uintptr_t)state | (uintptr_t)mask) & 15)
+        return fail(CRL_ERR_ARG, "crl_blokus_placement_mask: state and mask must be 16-byte aligned");
+    if ((uintptr_t)counts & 3) return fail(CRL_ERR_ARG, "crl_blokus_placement_mask: counts must be 4-byte aligned");
+    return launch("blokus_placement_mask_kernel", blokus_placement_mask_kernel, {blocks_for(B, BLK_WARPS), 32 * BLK_WARPS},
+                  stream, (const uint4 *)state, (uint4 *)mask, counts, B, player, frame, flags);
+}
+
+int crl_blokus_placement_to_action(const void *state, int player, int frame, const int32_t *placements, int32_t *actions,
+                                   int64_t B, int flags, crl_stream_t stream) {
+    if (!state || !placements || !actions || B < 0 || player > 3)
+        return fail(CRL_ERR_ARG, "crl_blokus_placement_to_action: bad argument");
+    if (frame != 0 && frame != 1) return fail(CRL_ERR_ARG, "crl_blokus_placement_to_action: frame must be 0 or 1");
+    if (B == 0) return CRL_OK;
+    if ((uintptr_t)state & 15) return fail(CRL_ERR_ARG, "crl_blokus_placement_to_action: state must be 16-byte aligned");
+    if (((uintptr_t)placements | (uintptr_t)actions) & 3)
+        return fail(CRL_ERR_ARG, "crl_blokus_placement_to_action: placements and actions must be 4-byte aligned");
+    static const BlkRotTab rot = [] {
+        BlkRotTab t = {};
+        for (int q = 0; q < 4; q++)
+            for (int s = 0; s < BLK_NSHAPE; s++) t.img[q][s] = (uint8_t)BLK_HOST_SHAPE_ROT[s][q];
+        return t;
+    }();
+    return launch("blokus_placement_to_action_kernel", blokus_placement_to_action_kernel,
+                  {blocks_for(B, BLK_WARPS), 32 * BLK_WARPS}, stream, (const uint4 *)state, placements, actions, B, player,
+                  frame, flags, rot);
+}
+
+int crl_blokus_shape_table(int32_t *shape_piece, int32_t *shape_cells, int32_t *shape_rotation, int32_t *action_shape) {
+    for (int s = 0; s < BLK_NSHAPE; s++) {
+        if (shape_piece) shape_piece[s] = BLK_HOST_SHAPE_PIECE[s];
+        for (int i = 0; i < 10; i++)
+            if (shape_cells) shape_cells[10 * s + i] = BLK_HOST_SHAPE_CELLS[s][i >> 1][i & 1];
+        for (int q = 0; q < 4; q++)
+            if (shape_rotation) shape_rotation[4 * s + q] = BLK_HOST_SHAPE_ROT[s][q];
+    }
+    for (int i = 0; i < BLK_NPIECE * 40 * 3; i++)
+        if (action_shape) action_shape[i] = (&BLK_HOST_ACTION_SHAPE[0][0][0])[i];
+    return BLK_NSHAPE;
+}
+
+}  // extern "C"

@@ -243,7 +243,46 @@ def emit(path):
     for _ in range(32):
         L.append("    {0u, 0u, 0u, 0u},")
     L.append("};")
+    emit_host_tables(L, shapes, piece_id0, ids)
     open(path, "w").write("\n".join(L) + "\n")
+
+
+# Rotation q of the board frame into player q's observation frame (np.rot90(k=-q)) on cell offsets:
+# (x, y) -> (19 - y, x), (19 - x, 19 - y), (y, 19 - x) for q = 1, 2, 3, i.e. these maps up to a translation.
+ROT_FRAME = [lambda x, y: (x, y), lambda x, y: (-y, x), lambda x, y: (-x, -y), lambda x, y: (y, -x)]
+
+
+def emit_host_tables(L, shapes, piece_id0, ids):
+    """Host-only copies for crl_blokus_shape_table and the placement launchers: plain `static const` arrays, so the
+    device code (and its constant banks) never sees them."""
+    index = {key: i for i, key in enumerate(shapes)}
+    L.append("// ---- host only (crl_blokus_shape_table, include/colosseum_b200_placement.h): no device storage")
+    L.append("// shape -> piece")
+    L.append("static const int8_t BLK_HOST_SHAPE_PIECE[BLK_NSHAPE] = {" + ", ".join(str(p) for p, _ in shapes) + "};")
+    L.append("// shape -> its cells (dx, dy), -1 past the shape's size")
+    L.append("static const int8_t BLK_HOST_SHAPE_CELLS[BLK_NSHAPE][5][2] = {")
+    for _, cells in shapes:
+        cl = [list(c) for c in cells] + [[-1, -1]] * (5 - len(cells))
+        L.append("    {" + ", ".join("{%d, %d}" % tuple(c) for c in cl) + "},")
+    L.append("};")
+    L.append("// shape -> its image in player q's rotated frame, q = 0..3")
+    L.append("static const int8_t BLK_HOST_SHAPE_ROT[BLK_NSHAPE][4] = {")
+    for p, cells in shapes:
+        img = []
+        for q in range(4):
+            rc = [ROT_FRAME[q](x, y) for x, y in cells]
+            mx, my = min(x for x, _ in rc), min(y for _, y in rc)
+            img.append(index[(p, tuple(sorted((x - mx, y - my) for x, y in rc)))])
+        L.append("    {" + ", ".join(map(str, img)) + "},")
+    L.append("};")
+    L.append("// (piece, o * 5 + k) -> (shape, dx, dy) of the id's orientation and of the shape cell on the anchor; -1 if k >= size")
+    L.append("static const int8_t BLK_HOST_ACTION_SHAPE[BLK_NPIECE][40][3] = {")
+    for p in range(len(piece_id0) - 1):
+        row = [[-1, -1, -1] for _ in range(40)]
+        for s, dx, dy, ok in ids[piece_id0[p]:piece_id0[p + 1]]:
+            row[ok] = [s, dx, dy]
+        L.append("    {" + ", ".join("{%d, %d, %d}" % tuple(v) for v in row) + "},")
+    L.append("};")
 
 
 if __name__ == "__main__":

@@ -129,6 +129,15 @@ class SingleAgentTurnVectorEnv:
         counts, ids = venv.valid_actions()           # Blokus: the seat's lists (perspective: in the rotated frame)
         obs, reward, done, info = venv.step(actions)  # reward int8 [B]; done uint8 [B]
 
+    With action_space="placement" (Blokus only) the learner acts on the fixed space of 36 400 placements
+    (colosseumrl_b200.blokus: p = shape * 400 + y * 20 + x) instead of the ragged id lists:
+
+        venv = SingleAgentTurnVectorEnv(BatchedBlokusEnvironment(batch=1024), seat=1, perspective=True,
+                                        action_space="placement")
+        counts, mask = venv.valid_actions()          # bool [B, 36 400], in the seat's frame
+        logits = logits.masked_fill(~mask, float("-inf"))
+        obs, reward, done, info = venv.step(placements)   # int32 [B]; an illegal placement: info["illegal"], a pass
+
     The rule is this engine's definition (include/colosseum_b200_learner.h).  Every returned game is the learner's
     turn; `done` marks the step in which a game finished, and that game has already been restarted (and played up to
     the learner's turn), so the observation describes the game the next action applies to.  reward: Tic Tac Toe +1 /
@@ -137,7 +146,7 @@ class SingleAgentTurnVectorEnv:
     "scores" (uint8 [B, 4], the finished game's).  The opponents' Philox step is a counter kept here (reset() sets it to
     0, and reset() itself is step 0)."""
 
-    def __init__(self, env, seat: int = 0, perspective: bool = False):
+    def __init__(self, env, seat: int = 0, perspective: bool = False, action_space: str = "id"):
         if not hasattr(env, "advance"):
             raise TypeError("SingleAgentTurnVectorEnv needs a Tic Tac Toe or Blokus environment")
         if not 0 <= seat < env.max_players:
@@ -145,7 +154,12 @@ class SingleAgentTurnVectorEnv:
         self.blokus = hasattr(env, "player_perspective_valid_actions")
         if perspective and not self.blokus:
             raise ValueError("perspective=True exists for Blokus only")
+        if action_space not in ("id", "placement"):
+            raise ValueError('action_space must be "id" or "placement"')
+        if action_space == "placement" and not self.blokus:
+            raise ValueError('action_space="placement" exists for Blokus only')
         self.env, self.seat, self.perspective = env, int(seat), bool(perspective)
+        self.action_space = action_space
         self.state, self.t = None, 0
 
     @property
@@ -162,8 +176,13 @@ class SingleAgentTurnVectorEnv:
         return self._observe()
 
     def valid_actions(self):
-        """Tic Tac Toe: the empty-cell mask int32 [B]; Blokus: (counts, ids) of the seat (perspective=True: rotated).
-        Fresh tensors: the next step() does not change them."""
+        """Tic Tac Toe: the empty-cell mask int32 [B]; Blokus: (counts, ids) of the seat (perspective=True: rotated), or
+        with action_space="placement" (counts, bool mask [B, 36 400]) of its legal placements.  Fresh tensors: the next
+        step() does not change them."""
+        if self.action_space == "placement":
+            from .blokus import placement_mask
+            counts, words = self.env.valid_placements(self.state, self.seat, self.perspective)
+            return counts, placement_mask(words)
         if not self.blokus:
             return self.env.valid_actions(self.state).clone()     # (the cached mask is rewritten by the next advance)
         if self.perspective:
@@ -172,8 +191,12 @@ class SingleAgentTurnVectorEnv:
 
     def step(self, actions):
         """actions: the learner's, int8 [B] cells (Tic Tac Toe) or int32 [B] ids (Blokus; perspective=True: in the
-        seat's rotated frame).  Returns (observation, reward int8 [B], done uint8 [B], info)."""
-        if self.perspective:
+        seat's rotated frame), or int32 [B] placements with action_space="placement" (one conversion launch to the
+        canonical ids; an illegal placement is reported in info["illegal"] and played as a pass).  Returns
+        (observation, reward int8 [B], done uint8 [B], info)."""
+        if self.action_space == "placement":
+            actions = self.env.placements_to_actions(self.state, actions, self.seat, self.perspective)
+        elif self.perspective:
             from .blokus import player_perspective_action_to_real
             actions = player_perspective_action_to_real(self.env._dev(actions, torch.int32), self.seat)
         rec = self.env.advance(self.state, actions, self.seat, self.t)

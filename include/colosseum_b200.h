@@ -260,4 +260,6 @@ int crl_blokus_pack(void *state, const int8_t *board, const uint8_t *pieces, con
 #include "colosseum_b200_tron_policy.h"
 /* one learner seat against device-side random opponents (Tic Tac Toe, Blokus) */
 #include "colosseum_b200_learner.h"
+/* Blokus placements: a fixed action space with legality masks, and placement -> action id */
+#include "colosseum_b200_placement.h"
 #endif

@@ -13,7 +13,7 @@ for mode in ${1:-address thread}; do
   CRL_HOSTSIM_SANITIZE=$mode python -c "import sys; sys.path.insert(0, 'tests/hostsim'); import build_hostsim; print(build_hostsim.build())"
   log=profiles/r02_hostsim_$tag.log
   echo "# $mode sanitizer on the SIMT emulator: pytest tests/test_hostsim_*.py tests/test_tron_planes.py tests/test_api_contract.py  ($(date -u +%FT%TZ))" > $log
-  CRL_HOSTSIM_SANITIZE=$mode LD_PRELOAD=$rt python -m pytest tests/test_hostsim_tron.py tests/test_hostsim_ttt.py tests/test_hostsim_blokus.py tests/test_hostsim_blokus_rollout.py tests/test_hostsim_tron_avoid.py tests/test_hostsim_learner.py tests/test_tron_planes.py tests/test_api_contract.py -m "not gpu" -q -x -p no:cacheprovider >> $log 2>&1
+  CRL_HOSTSIM_SANITIZE=$mode LD_PRELOAD=$rt python -m pytest tests/test_hostsim_tron.py tests/test_hostsim_ttt.py tests/test_hostsim_blokus.py tests/test_hostsim_blokus_rollout.py tests/test_hostsim_tron_avoid.py tests/test_hostsim_learner.py tests/test_hostsim_blokus_placement.py tests/test_tron_planes.py tests/test_api_contract.py -m "not gpu" -q -x -p no:cacheprovider >> $log 2>&1
   echo "exit code $?" >> $log
   grep -c -E "ERROR: AddressSanitizer|WARNING: ThreadSanitizer|runtime error" $log | sed "s/^/sanitizer reports: /" >> $log
   tail -4 $log
